@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference algorithm on host cores
     python bench.py --config C1|C2|C3|C4|C5 [--c5-k 100000] [--c5-mode topk_nms|nms_all]
+    python bench.py ... --dump-outputs DIR                   # also save the last timed step's outputs (.npy)
 
 A "step" is one pass of the hot path over one synthetic batch: calculate_rpn_actual_outputs
 (target assignment) + generate_proposals (decode, clip, top-6000, NMS 300 @ 0.7) for the batch one
@@ -390,6 +391,9 @@ def run_ours(args):
     sampler.sample()                        # the GPU is still working through the queue
     barrier()
     clocks = sampler.result()
+    if args.dump_outputs and rank == 0:
+        # the buffers of the last timed step, read now: the passes below write into the same sets
+        dump_outputs(args.dump_outputs, sets[(W + K - 1) % SETS], rpn)
     ms = e0.elapsed_time(e1)
     if world > 1:
         t = torch.tensor([ms], device=dev)
@@ -653,6 +657,19 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+def dump_outputs(out_dir, s, rpn):
+    """Write the arrays a caller of the timed path receives, one DIR/<name>.npy each (float32, integer
+    outputs as float64, which holds every int32 exactly).  Every config's outputs fit in 64 MB whole."""
+    names = ({"deltas": "bbox_deltas", "labels": "bbox_labels", "pb": "proposal_boxes", "ps": "proposal_scores",
+              "pv": "proposal_valid", "pk": "proposal_keep"} if rpn else
+             {"pb": "nmsed_boxes", "ps": "nmsed_scores", "pc": "nmsed_classes", "pv": "valid_detections",
+              "pk": "keep_indices"})
+    os.makedirs(out_dir, exist_ok=True)
+    for key, name in names.items():
+        a = s[key].cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
+
+
 def e2e_rpn(args, wl, lib, _lib, h, hp, anchors, np_sets, tcfg, pcfg, wall, world, rank, dev, K):
     """HostPipeline (tfrpn_pipeline_* C ABI) with the slots' page-locked blocks as the caller's buffers."""
     import torch
@@ -804,7 +821,11 @@ def main():
     ap.add_argument("--c5-mode", default="topk_nms", choices=["topk_nms", "nms_all"])
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:
