@@ -7,12 +7,13 @@
 // Order: every entry gets the unique 64-bit composite  (orderable(score) << 32) | ~index , so
 // "larger composite" == "higher score, and among equal scores the LOWER index" -- the order of
 // tf.nn.top_k and the order in which TF's NMS pops candidates ([TF-internal]; ties documented in
-// the oracle).  NMS is lazy: it consumes candidates in BATCHES of 1024 ranks and usually stops
+// the oracle).  NMS is lazy: it consumes candidates in BATCHES of at most 1024 ranks and usually stops
 // (max_output_size kept) inside the first batch, so the other ~5000 of the pre-NMS top-6000 are
-// never sorted, gathered or decoded.  Per batch, inside the CTA:
-//   1 radix SELECT (MSB first, 8 bits/pass, early exit) of the composite at rank `hi`
-//   2 unordered COMPACTION of the entries with rank in [lo, hi) into shared memory
-//   3 BITONIC SORT of those <= 1024 composites, one per thread (shuffles below stride 32)
+// never sorted, gathered or decoded.  Per batch, inside the CTA (proposal_kernel):
+//   1 SELECT a threshold tau with 11-bit histograms (the first one built while the keys are staged):
+//     the batch is every remaining composite >= tau, between 768 and 1024 of them (fewer: all that remain)
+//   2 the batch's entries, from a short candidate list the select copied out, or one compaction sweep
+//   3 COUNTING SORT on 11 key bits, entries of a bin ranked by comparison (bitonic network for long bins)
 //   4 top-k outputs, or greedy NMS rounds of 128 candidates: test against the kept list, build
 //     predecessor masks inside the round, resolve them in one warp with ballots.
 //   In the fused mode boxes are decoded (+clipped) on the fly, for the examined candidates only.
@@ -117,11 +118,19 @@ struct PropParams {
     int nms_rows, mask_words;
 };
 
+// proposal_kernel front end (see there): 11-bit digits, 2048-bin shared histograms scanned two bins per thread
+constexpr int SEL_BITS = 11;
+constexpr int SEL_NB = 1 << SEL_BITS;
+constexpr int SEL_FLOOR = BATCH * 3 / 4;   // a batch may end at a histogram bin edge once it holds this many entries
+constexpr int SEL_LIST = 2 * BATCH;        // candidate-list capacity: the sort buffer
+constexpr int SEG_MAX = 32;                // longest counting-sort bin ordered by comparisons; longer -> bitonic network
+
 struct PropShared {
-    unsigned int hist[256];
-    unsigned int wtot[PR_WARPS];
-    unsigned int digit, remaining, bin_count;
-    unsigned int count;
+    unsigned int wtot[PR_WARPS], wmax[PR_WARPS];
+    unsigned int digit, excl, bin_count;
+    unsigned int count;      // entries above the score threshold
+    unsigned int lcount;     // candidate-list cursor
+    unsigned int kmax;       // largest key of the image
     int nk;
     int nalive;
 };
@@ -140,20 +149,24 @@ __device__ __forceinline__ unsigned long long make_comp(uint32_t key, int i) {
     return ((unsigned long long)key << 32) | (unsigned long long)(0xFFFFFFFFu - (uint32_t)i);
 }
 
-// block-wide sum of one unsigned per thread
-__device__ __forceinline__ unsigned int block_sum(unsigned int v, PropShared* sh) {
-    unsigned int incl = (unsigned int)warp_incl_scan((int)v);
-    if (lane_id() == 31) sh->wtot[warp_id()] = incl;
+// Block-wide scan of SEL_NB histogram bins from the top: thread t owns bins SEL_NB-1-2t (c0) and SEL_NB-2-2t (c1).
+// excl = entries in the bins above c0, total = all entries, cmax = the fullest bin.  One barrier inside; sh->wtot /
+// sh->wmax may be rewritten only after another barrier.
+__device__ __forceinline__ void hist_scan_desc(const unsigned int* hist, unsigned& c0, unsigned& c1, unsigned& excl,
+                                               unsigned& total, unsigned& cmax, PropShared* sh) {
+    const int t = threadIdx.x, lane = lane_id(), warp = warp_id();
+    c0 = hist[SEL_NB - 1 - 2 * t];
+    c1 = hist[SEL_NB - 2 - 2 * t];
+    const unsigned s = c0 + c1;
+    const unsigned incl = (unsigned)warp_incl_scan((int)s);
+    const unsigned m = __reduce_max_sync(0xffffffffu, max(c0, c1));
+    if (lane == 31) { sh->wtot[warp] = incl; sh->wmax[warp] = m; }
     __syncthreads();
-    if (warp_id() == 0) {
-        unsigned int w = sh->wtot[lane_id()];
-        unsigned int wi = (unsigned int)warp_incl_scan((int)w);
-        if (lane_id() == 31) sh->count = wi;
-    }
-    __syncthreads();
-    unsigned int r = sh->count;
-    __syncthreads();
-    return r;
+    const unsigned w = sh->wtot[lane];
+    const unsigned wi = (unsigned)warp_incl_scan((int)w);
+    total = __shfl_sync(0xffffffffu, wi, 31);
+    excl = __shfl_sync(0xffffffffu, wi - w, warp) + incl - s;
+    cmax = __reduce_max_sync(0xffffffffu, sh->wmax[lane]);
 }
 
 // TF CombinedNonMaxSuppression IOU on canonicalised boxes ([TF-internal]); c = (ymin,xmin,ymax,xmax).
@@ -258,7 +271,7 @@ __global__ void __launch_bounds__(PR_THREADS, 1) proposal_kernel(PropParams p) {
     const float4* anc = p.anchors + (p.anchors_batched ? (long long)b * SN : 0LL);
     const int* remap = p.remap ? p.remap + (long long)b * SN : nullptr;
 
-    unsigned long long* sortbuf = reinterpret_cast<unsigned long long*>(smem4);   // [2 * BATCH]
+    unsigned long long* sortbuf = reinterpret_cast<unsigned long long*>(smem4);   // [2 * BATCH] list, then the batch
     uint32_t* sidx = reinterpret_cast<uint32_t*>(sortbuf + 2 * BATCH);            // [BATCH] sorted indices
     float4* kbox = reinterpret_cast<float4*>(sidx + BATCH);                       // [mo_pad]
     float4* cbox = kbox + p.mo_pad;                                               // [NMS_CHUNK]
@@ -267,18 +280,47 @@ __global__ void __launch_bounds__(PR_THREADS, 1) proposal_kernel(PropParams p) {
     unsigned int* alive = reinterpret_cast<unsigned int*>(carea + NMS_CHUNK);     // [NMS_CHUNK]
     int* slot = reinterpret_cast<int*>(alive + NMS_CHUNK);                        // [NMS_CHUNK]
     unsigned int* mask32 = reinterpret_cast<unsigned int*>(slot + NMS_CHUNK);       // [NMS_CHUNK][4]
-    uint32_t* skeys = mask32 + NMS_CHUNK * 4;                                     // [N] when staged
+    unsigned int* hist = mask32 + NMS_CHUNK * 4;                                  // [SEL_NB]
+    uint32_t* skeys = hist + SEL_NB;                                              // [N] when staged
 
-    // ---- phase 0: stage keys, count entries above the score threshold ---------------------------
-    unsigned int my_valid = 0;
-    for (int i = tid; i < N; i += PR_THREADS) {
-        uint32_t key = score_key(scores[i], p.use_sthr, p.score_threshold);
-        if (p.staged) skeys[i] = key;
-        my_valid += (key != 0u) ? 1u : 0u;
+    // Entries at or below the score threshold (key 0) can never be consumed (K <= M below), so with a threshold
+    // they take no part in any batch: composites with key 0 are <= cmin.
+    const unsigned long long cmin = p.use_sthr ? 0xFFFFFFFFull : 0ull;
+
+    // ---- phase 0: stage keys; count entries above the score threshold, the largest key and the first select
+    //      histogram (key bits [31:21]) in the same sweep, four loads in flight per thread --------------------
+    hist[2 * tid] = 0u;
+    hist[2 * tid + 1] = 0u;
+    if (tid == 0) { sh.count = 0u; sh.kmax = 0u; }
+    __syncthreads();
+    unsigned int my_valid = 0, my_max = 0;
+    for (int base = 0; base < N; base += 4 * PR_THREADS) {
+        float sc[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const int i = base + u * PR_THREADS + tid;
+            sc[u] = i < N ? __ldg(scores + i) : 0.0f;
+        }
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const int i = base + u * PR_THREADS + tid;
+            if (i < N) {
+                const uint32_t key = score_key(sc[u], p.use_sthr, p.score_threshold);
+                if (p.staged) skeys[i] = key;
+                my_max = max(my_max, key);
+                if (key != 0u || !p.use_sthr) {
+                    ++my_valid;
+                    atomicAdd(&hist[key >> (32 - SEL_BITS)], 1u);
+                }
+            }
+        }
     }
-    int M = N;
-    if (p.use_sthr) M = (int)block_sum(my_valid, &sh);
-    else __syncthreads();
+    my_valid = __reduce_add_sync(0xffffffffu, my_valid);
+    my_max = __reduce_max_sync(0xffffffffu, my_max);
+    if (lane == 0) { atomicAdd(&sh.count, my_valid); atomicMax(&sh.kmax, my_max); }
+    __syncthreads();
+    const int M = (int)sh.count;   // N without a score threshold
+    const uint32_t kmax = sh.kmax;
     const int K = min(p.k, M);  // ranks that may be consumed
     PH(1);
     int nkept = 0;
@@ -288,96 +330,154 @@ __global__ void __launch_bounds__(PR_THREADS, 1) proposal_kernel(PropParams p) {
         return p.staged ? skeys[i] : score_key(scores[i], p.use_sthr, p.score_threshold);
     };
 
-    // rule "rank < r":  (comp >> shift) >= P   (the lo rule of the first batch selects nothing)
-    int lo_shift = 0;
-    unsigned long long lo_P = ~0ull;
+    // Batches by threshold: a batch is every eligible entry with composite >= tau, where tau is a histogram bin
+    // edge chosen so that the batch holds at most BATCH entries, and at least SEL_FLOOR unless it holds every
+    // eligible entry.  Entries of earlier batches (composite >= lo_tau) are no longer eligible.  The batch is
+    // ordered in full, so its first K - lo ranks end exactly at rank K.
+    unsigned long long lo_tau = 0ull;
     bool have_lo = false;
-
-    for (int lo = 0; lo < K; lo += BATCH) {
-        const int hi = min(lo + BATCH, K);
-        // ---- 1. radix select of the composite at rank hi --------------------------------------
-        int shift = 0;
-        unsigned long long P = 0ull;          // hi == N: everything is selected
-        if (hi < N) {
-            unsigned long long prefix = 0ull;
-            unsigned int r = (unsigned int)hi;
-            shift = 56;
-            for (int pass = 0; pass < 8; ++pass) {
-                if (tid < 256) sh.hist[tid] = 0u;
-                __syncthreads();
-                const unsigned long long himask = pass == 0 ? 0ull : (~0ull << (shift + 8));
-                for (int i = tid; i < N; i += PR_THREADS) {
-                    const unsigned long long c = make_comp(key_at(i), i);
-                    if (((c ^ prefix) & himask) == 0ull) atomicAdd(&sh.hist[(unsigned)(c >> shift) & 255u], 1u);
+    for (int lo = 0; lo < K;) {
+        auto eligible = [&](unsigned long long c) -> bool { return c > cmin && (!have_lo || c < lo_tau); };
+        // ---- 1. select tau: 11-bit digits from the top of the composite, refined inside the bin that holds
+        //      rank BATCH.  Once the eligible entries >= the bin's lower edge fit SEL_LIST, the next full sweep
+        //      also copies them into sortbuf and every later pass (and the batch) reads only that list. ----------
+        unsigned long long tau = 0ull, prefix = 0ull;   // tau 0: every eligible entry
+        int top = 63;                                   // digit bits [top - 10, top] below the common prefix
+        unsigned int r = BATCH;                         // rank of the boundary among entries matching `prefix`
+        int nl = -1;                                    // entries in the list (-1: none, sweep all N)
+        bool listing = false;
+        for (int pass = 0;; ++pass) {
+            const int shift = max(top - (SEL_BITS - 1), 0);
+            const unsigned int dmask = (2u << (top - shift)) - 1u;
+            const unsigned long long himask = top >= 63 ? 0ull : (~0ull << (top + 1));
+            if (nl >= 0) {
+                for (int q = tid; q < nl; q += PR_THREADS) {
+                    const unsigned long long c = sortbuf[q];
+                    if (((c ^ prefix) & himask) == 0ull) atomicAdd(&hist[(unsigned)(c >> shift) & dmask], 1u);
                 }
-                __syncthreads();
-                if (tid < 32) {   // lane l owns digits [248-8l, 255-8l], scanned from the top
-                    const int top = 255 - 8 * lane;
-                    unsigned int s = 0;
-#pragma unroll
-                    for (int d = 0; d < 8; ++d) s += sh.hist[top - d];
-                    const unsigned int incl = (unsigned int)warp_incl_scan((int)s);
-                    const unsigned int excl = incl - s;
-                    if (excl < r && r <= incl) {
-                        unsigned int acc = excl;
-                        for (int d = 0; d < 8; ++d) {
-                            const unsigned int c = sh.hist[top - d];
-                            if (acc + c >= r) {
-                                sh.digit = (unsigned)(top - d);
-                                sh.remaining = r - acc;
-                                sh.bin_count = c;
-                                break;
-                            }
-                            acc += c;
+            } else if (pass > 0 || have_lo) {           // (the first batch's first histogram comes from phase 0)
+                for (int base = 0; base < N; base += PR_THREADS) {
+                    const int i = base + tid;
+                    unsigned long long c = 0ull;
+                    bool in = false;                    // eligible and >= prefix: above the bin, or in it
+                    if (i < N) {
+                        c = make_comp(key_at(i), i);
+                        in = eligible(c) && c >= prefix;
+                    }
+                    if (in && ((c ^ prefix) & himask) == 0ull) atomicAdd(&hist[(unsigned)(c >> shift) & dmask], 1u);
+                    if (listing) {
+                        const unsigned bal = __ballot_sync(0xffffffffu, in);
+                        if (bal != 0u) {
+                            unsigned int pos0 = 0;
+                            if (lane == __ffs(bal) - 1) pos0 = atomicAdd(&sh.lcount, (unsigned)__popc(bal));
+                            pos0 = __shfl_sync(0xffffffffu, pos0, __ffs(bal) - 1);
+                            if (in) sortbuf[pos0 + __popc(bal & ((1u << lane) - 1u))] = c;
                         }
                     }
                 }
-                __syncthreads();
-                prefix |= (unsigned long long)sh.digit << shift;
-                r = sh.remaining;
-                const bool done = (sh.bin_count == r);   // the whole bin is taken: stop refining
-                __syncthreads();
-                if (done || pass == 7) break;
-                shift -= 8;
             }
-            P = prefix >> shift;
+            __syncthreads();                            // histogram (and list) complete
+            if (listing) nl = (int)sh.lcount;
+            unsigned c0, c1, ex0, total, cmax;
+            hist_scan_desc(hist, c0, c1, ex0, total, cmax, &sh);
+            hist[SEL_NB - 1 - 2 * tid] = 0u;             // own bins, for the next histogram (after the barrier below)
+            hist[SEL_NB - 2 - 2 * tid] = 0u;
+            if (ex0 < r && r <= ex0 + c0 + c1) {
+                const bool upper = r <= ex0 + c0;
+                sh.digit = (unsigned)(SEL_NB - 1 - 2 * tid) - (upper ? 0u : 1u);
+                sh.excl = upper ? ex0 : ex0 + c0;
+                sh.bin_count = upper ? c0 : c1;
+            }
+            if (tid == 0) sh.lcount = 0u;
+            __syncthreads();
+            if (total < r) break;                       // (first pass only) fewer than BATCH eligible entries: all of them
+            const unsigned int d = sh.digit, ex = sh.excl, bc = sh.bin_count;
+            const unsigned long long edge = prefix | ((unsigned long long)d << shift);   // lower edge of the boundary bin
+            const unsigned int above = BATCH - r + ex;  // eligible entries above the boundary bin
+            if (bc == r - ex) { tau = edge; break; }    // the whole bin makes exactly BATCH
+            if (above >= (unsigned)SEL_FLOOR) { tau = edge + (1ull << shift); break; }
+            listing = nl < 0 && above + bc <= (unsigned)SEL_LIST;
+            prefix = edge;
+            r -= ex;
+            top = shift - 1;                            // (shift == 0 cannot get here: its bins are single composites)
         }
         PH(2);
-        // ---- 2. compaction of ranks [lo, hi) (any order: composites are unique) -----------------
-        if (tid == 0) sh.count = 0u;
-        sortbuf[tid] = 0ull;                    // padding sorts last
-        __syncthreads();
-        for (int base = 0; base < N; base += PR_THREADS) {
-            const int i = base + tid;
-            bool take = false;
-            unsigned long long c = 0ull;
-            if (i < N) {
-                c = make_comp(key_at(i), i);
-                take = ((c >> shift) >= P) && !(have_lo && ((c >> lo_shift) >= lo_P));
+        // ---- 2. the batch: up to two list entries per thread (without a list, one compaction sweep makes it) ----
+        if (nl < 0) {
+            for (int base = 0; base < N; base += PR_THREADS) {
+                const int i = base + tid;
+                bool take = false;
+                unsigned long long c = 0ull;
+                if (i < N) {
+                    c = make_comp(key_at(i), i);
+                    take = eligible(c) && c >= tau;
+                }
+                const unsigned bal = __ballot_sync(0xffffffffu, take);
+                if (bal != 0u) {
+                    unsigned int pos0 = 0;
+                    if (lane == __ffs(bal) - 1) pos0 = atomicAdd(&sh.lcount, (unsigned)__popc(bal));
+                    pos0 = __shfl_sync(0xffffffffu, pos0, __ffs(bal) - 1);
+                    if (take) sortbuf[pos0 + __popc(bal & ((1u << lane) - 1u))] = c;
+                }
             }
-            const unsigned bal = __ballot_sync(0xffffffffu, take);
-            if (bal != 0u) {
-                unsigned int basepos = 0;
-                if (lane == __ffs(bal) - 1) basepos = atomicAdd(&sh.count, (unsigned)__popc(bal));
-                basepos = __shfl_sync(0xffffffffu, basepos, __ffs(bal) - 1);
-                if (take) sortbuf[basepos + __popc(bal & ((1u << lane) - 1u))] = c;
-            }
+            __syncthreads();
+            nl = (int)sh.lcount;
         }
-        __syncthreads();
+        // list entries are eligible and >= tau's bin edge or better; composites of entries are > 0
+        const unsigned long long e0 = tid < nl ? sortbuf[tid] : 0ull;
+        const unsigned long long e1 = tid + BATCH < nl ? sortbuf[tid + BATCH] : 0ull;
+        const bool m0 = e0 != 0ull && e0 >= tau, m1 = e1 != 0ull && e1 >= tau;
         PH(3);
-        // ---- 3. sort: thread t gets the composite of rank lo + t ---------------------------------
-        unsigned long long mine = sortbuf[tid];
+        // ---- 3. order the batch: counting sort on the 11 key bits below the common prefix of its key range
+        //      [key(tau), upper bound]; a bin's entries find their place by comparing composites within it ---------
+        const uint32_t khi = have_lo ? (uint32_t)(lo_tau >> 32) : kmax, kdiff = khi ^ (uint32_t)(tau >> 32);
+        const int sshift = kdiff ? max(31 - __clz(kdiff) - (SEL_BITS - 1), 0) : 0;
+        unsigned d0 = 0, d1 = 0, s0 = 0, s1 = 0;
+        if (m0) { d0 = ((uint32_t)(e0 >> 32) >> sshift) & (SEL_NB - 1); s0 = atomicAdd(&hist[d0], 1u); }
+        if (m1) { d1 = ((uint32_t)(e1 >> 32) >> sshift) & (SEL_NB - 1); s1 = atomicAdd(&hist[d1], 1u); }
+        __syncthreads();                                // bin counts complete; the list has been read
+        unsigned c0, c1, ex0, total, cmax;
+        hist_scan_desc(hist, c0, c1, ex0, total, cmax, &sh);
+        hist[SEL_NB - 1 - 2 * tid] = (ex0 << 16) | c0;  // (first position, count) of the own bins
+        hist[SEL_NB - 2 - 2 * tid] = ((ex0 + c0) << 16) | c1;
         __syncthreads();
-        mine = bitonic_sort_desc(mine, sortbuf);
-        const int nb = hi - lo;                 // entries in this batch
+        const int nb_all = (int)total;                  // entries of this batch, <= BATCH
+        unsigned long long* bybin = sortbuf;            // [BATCH] the batch grouped by bin
+        unsigned long long* ranked = sortbuf + BATCH;   // [BATCH] the batch in rank order
+        if (m0) bybin[(hist[d0] >> 16) + s0] = e0;
+        if (m1) bybin[(hist[d1] >> 16) + s1] = e1;
+        __syncthreads();
+        unsigned long long mine;
+        if (cmax <= (unsigned)SEG_MAX) {
+            auto place = [&](unsigned long long e, unsigned d) {
+                const unsigned hv = hist[d], first = hv >> 16, n = hv & 0xFFFFu;
+                unsigned gt = 0;
+                for (unsigned q = 0; q < n; ++q) gt += bybin[first + q] > e ? 1u : 0u;
+                ranked[first + gt] = e;
+            };
+            if (m0) place(e0, d0);
+            if (m1) place(e1, d1);
+            __syncthreads();
+            mine = tid < nb_all ? ranked[tid] : 0ull;
+        } else {                                        // long bins (tie groups, clustered scores): bitonic network
+            mine = tid < nb_all ? bybin[tid] : 0ull;    // padding sorts last
+            __syncthreads();
+            mine = bitonic_sort_desc(mine, sortbuf);
+        }
+        hist[2 * tid] = 0u;                             // for the next batch: its first histogram follows a barrier
+        hist[2 * tid + 1] = 0u;
+        const int blo = lo;                             // thread t holds rank blo + t
+        const int nb = min(nb_all, K - lo);             // entries of this batch that may be consumed
+        lo += nb_all;
+        lo_tau = tau;
+        have_lo = true;
         PH(4);
         const uint32_t my_i = 0xFFFFFFFFu - (uint32_t)(mine & 0xFFFFFFFFull);
-        lo_shift = shift; lo_P = P; have_lo = true;
 
         // ---- 4a. top-k outputs (predictor.py:58-60) -------------------------------------------
         if (p.mode == MODE_TOPK) {
             if (tid < nb) {
-                const long long o = (long long)b * p.k + lo + tid;
+                const long long o = (long long)b * p.k + blo + tid;
                 p.values[o] = scores[my_i];
                 p.indices[o] = remap ? remap[my_i] : (int)my_i;
                 if (p.gathered) {
@@ -1416,6 +1516,7 @@ static size_t prop_smem_bytes(int n_staged, int max_out) {
     s += (size_t)BATCH * 4;                         // sidx
     s += (size_t)(max_out + NMS_CHUNK) * (16 + 4);  // kbox+cbox, karea+carea
     s += (size_t)NMS_CHUNK * (4 + 4 + 16);          // alive, slot, mask16
+    s += (size_t)SEL_NB * 4;                        // select / counting-sort histogram
     s += (size_t)n_staged * 4;                      // staged score keys
     return s + 16;
 }
