@@ -53,6 +53,7 @@ int ensure_kernel_attributes(int device) {
     if (int rc = set_attributes_targets()) return rc;
     if (int rc = set_attributes_proposals()) return rc;
     if (int rc = set_attributes_boxmath()) return rc;
+    if (int rc = set_attributes_evaluate()) return rc;
     done[device] = true;
     return 0;
 }
@@ -156,6 +157,7 @@ extern "C" const char* tfrpn_kernel_name(int id) {
         case TFRPN_K_NMS_MASK: return "nms_mask_kernel";
         case TFRPN_K_NMS_SWEEP: return "nms_sweep_kernel";
         case TFRPN_K_LOSS: return "rpn_loss_partial_kernel";
+        case TFRPN_K_RECALL: return "recall_kernel";
         default: return "?";
     }
 }

@@ -43,6 +43,11 @@ class LossOut(C.Structure):
     _fields_ = [("reg_loss", C.c_float), ("cls_loss", C.c_float), ("n_pos", C.c_int32), ("n_cls", C.c_int32)]
 
 
+class RecallCfg(C.Structure):
+    _fields_ = [("n_thresholds", C.c_int32), ("thresholds", C.c_float * 16), ("n_limits", C.c_int32),
+                ("limits", C.c_int32 * 8), ("matching", C.c_int32), ("reserved", C.c_int32)]
+
+
 class StepBuffers(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("gt_boxes", "gt_labels", "rpn_reg", "rpn_cls", "deltas", "labels",
                                           "out_boxes", "out_scores", "valid", "keep_idx")]
@@ -50,7 +55,7 @@ class StepBuffers(C.Structure):
 
 P = C.c_void_p
 I = C.c_int
-KERNEL_IDS = 8   # TFRPN_K_COUNT of include/tfrpn.h
+KERNEL_IDS = 9   # TFRPN_K_COUNT of include/tfrpn.h
 # name -> (restype, argtypes); must list every symbol include/tfrpn.h declares
 PROTOTYPES = {
     "tfrpn_version": (I, []),
@@ -100,6 +105,7 @@ PROTOTYPES = {
     "tfrpn_pipeline_destroy": (I, [P]),
     "tfrpn_host_alloc": (I, [C.POINTER(P), C.c_size_t]),
     "tfrpn_host_free": (I, [P]),
+    "tfrpn_proposal_recall": (I, [P, P, P, P, P, I, I, I, C.POINTER(RecallCfg), P, P, P]),
 }
 
 _lib = None
