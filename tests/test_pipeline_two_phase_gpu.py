@@ -43,29 +43,38 @@ class Env:
                 os.environ[k] = v
 
 
-def want_for(anchors_np, hp, gtb, gtl, reg, cls, seed, offset, image_offset):
+def want_for(anchors_np, hp, gtb, gtl, reg, cls, seed, offset, image_offset, pre_nms_topn=6000):
     B = gtb.shape[0]
     if CO.available():
         od, ol = CO.rpn_targets(anchors_np, gtb, gtl, hp, seed=seed, offset=offset, image_offset=image_offset)
-        wb, ws, wv, wk = CO.proposals(reg.reshape(B, -1, 4), cls.reshape(B, -1), anchors_np, hp, 6000)
+        wb, ws, wv, wk = CO.proposals(reg.reshape(B, -1, 4), cls.reshape(B, -1), anchors_np, hp, pre_nms_topn)
     else:
         od, ol = O.calculate_rpn_actual_outputs(anchors_np, gtb, gtl, hp, seed=seed, offset=offset, image_offset=image_offset)
-        wb, ws, wv, wk = O.generate_proposals(reg, cls, anchors_np, hp, pre_nms_topn=6000)
+        wb, ws, wv, wk = O.generate_proposals(reg, cls, anchors_np, hp, pre_nms_topn=pre_nms_topn)
     return od, ol.reshape(B, -1), wb, ws, wv, wk
 
 
-def run_acquired(cuda_device, B, G, depth, steps, env):
+def synthetic_head(i, B):
+    from tfrpn import synthetic
+    return synthetic.head_outputs(np.random.default_rng(800 + i), B, 31, 31, 9)
+
+
+def run_acquired(cuda_device, B, G, depth, steps, env, pre_nms_topn=6000, head=synthetic_head):
+    """`steps` steps through acquired slots; head(i, B) gives step i's (rpn_reg, rpn_cls)"""
     from tfrpn import HostPipeline, synthetic
     hp = dict(O.get_hyper_params("vgg16"))
     anchors_np = O.generate_anchors(hp)
     with Env(**env):
-        pipe = HostPipeline(hp, depth=depth, device=cuda_device, pre_nms_topn=6000)
-    pending, copied = [], []
+        pipe = HostPipeline(hp, depth=depth, device=cuda_device, pre_nms_topn=pre_nms_topn)
+    # the slot views live apart from the pending items: a failure report shows check()'s argument, and the views'
+    # page-locked memory is freed by pipe.close() before the report is written
+    pending, copied, views = [], [], {}
     try:
         def check(item):
-            t, v, i, gtb, gtl, reg, cls = item
+            t, i, gtb, gtl, reg, cls = item
             pipe.wait(t)
-            od, ol, wb, ws, wv, wk = want_for(anchors_np, hp, gtb, gtl, reg, cls, 21, i, 5 * i)
+            v = views.pop(t)
+            od, ol, wb, ws, wv, wk = want_for(anchors_np, hp, gtb, gtl, reg, cls, 21, i, 5 * i, pre_nms_topn)
             assert bits_equal(v.labels.reshape(B, -1), ol) and close(v.deltas, od)
             assert np.array_equal(v.deltas != 0, od != 0)
             assert np.array_equal(v.valid, wv) and np.array_equal(v.keep_idx, wk)
@@ -73,12 +82,15 @@ def run_acquired(cuda_device, B, G, depth, steps, env):
             copied.append(pipe.last_copy_bytes())
         for i in range(steps):
             gtb, gtl = synthetic.gt_batch(np.random.default_rng(700 + i), B, G)
-            reg, cls = synthetic.head_outputs(np.random.default_rng(800 + i), B, 31, 31, 9)
+            reg, cls = head(i, B)
             if len(pending) == depth - 1:
                 check(pending.pop(0))
             v = pipe.acquire(B, G)
             v.gt_boxes[...] = gtb; v.gt_labels[...] = gtl; v.rpn_reg[...] = reg; v.rpn_cls[...] = cls
-            pending.append((pipe.submit(seed=21, offset=i, image_offset=5 * i), v, i, gtb, gtl, reg, cls))
+            v.out_boxes[...] = np.nan; v.out_scores[...] = np.nan; v.valid[...] = -7; v.keep_idx[...] = -7
+            t = pipe.submit(seed=21, offset=i, image_offset=5 * i)
+            views[t] = v
+            pending.append((t, i, gtb, gtl, reg, cls))
         while pending:
             check(pending.pop(0))
     finally:
@@ -228,6 +240,105 @@ def test_submit_arrays_stable_outputs_ring(cuda_device):
                 check(pending.pop(0))
             t, out = pipe.submit_arrays(gtb, gtl, reg, cls, out=outs[i % depth], seed=4, offset=i)
             pending.append((t, i, out, gtb, gtl, reg, cls))
+        while pending:
+            check(pending.pop(0))
+    finally:
+        pipe.close()
+
+
+# ---- adversarial scores and regressions ---------------------------------------------------------------------------
+
+def tie_scores(rng, B, name, N=8649):
+    """(B, N) scores made of tie groups (no -0 beside +0, no -inf: the oracle orders them like the kernels)"""
+    if name == "equal":
+        return np.full((B, N), 0.5, F32)
+    if name == "three":                       # tie groups across the batch floor, rank 1024 and the pre-NMS cap
+        s = np.full((B, N), 0.25, F32)
+        s[:, :700] = 0.75
+        s[:, 700:1100] = 0.5
+        return np.stack([r[rng.permutation(N)] for r in s])
+    if name == "one_bin_ulps":                # 16 distinct values inside one 11-bit bin
+        return (1.0 - 2.0 ** -20 * rng.uniform(0, 1, size=(B, N))).astype(F32)
+    if name == "coarse":                      # 65 values: tie groups of ~130 entries everywhere
+        return (np.round(rng.uniform(0, 1, size=(B, N)) * 64) / 64).astype(F32)
+    raise ValueError(name)
+
+
+TIE_LAYOUTS = ["three", "equal", "one_bin_ulps", "coarse"]
+
+
+def collapsed_head(i, B):
+    """Step i: rpn_cls from a tie layout, and rpn_reg that decodes a share of the anchors (all, 90 %, half or none,
+    by image) onto five boxes per image.  NMS then suppresses nearly everything, runs out of the gathered rows and
+    the image is redone; the other images finish inside them."""
+    hp = O.get_hyper_params("vgg16")
+    anchors = O.generate_anchors(hp)
+    N = anchors.shape[0]
+    rng = np.random.default_rng(300 + i)
+    cls = tie_scores(rng, B, TIE_LAYOUTS[i % len(TIE_LAYOUTS)])
+    reg = rng.normal(0, 0.5, size=(B, N, 4)).astype(F32)
+    c = rng.uniform(0.2, 0.8, size=(B, 5, 2))
+    sz = rng.uniform(0.1, 0.4, size=(B, 5, 2))
+    targets = np.clip(np.concatenate([c - sz / 2, c + sz / 2], -1), 0, 1).astype(F32)
+    onto = np.take_along_axis(targets, rng.integers(0, 5, size=(B, N, 1)).repeat(4, -1), axis=1)
+    deltas = CO.encode(anchors, onto) / np.asarray(hp["variances"], F32) + rng.normal(0, 0.002, size=(B, N, 4))
+    share = np.array([1.0, 0.9, 0.5, 0.0])[np.arange(B) % 4]
+    m = rng.uniform(size=(B, N)) < share[:, None]
+    reg[m] = deltas[m]
+    return reg.astype(F32).reshape(B, 31, 31, 36), cls.reshape(B, 31, 31, 9)
+
+
+TWO_PHASE_PATHS = {
+    "host": {},
+    "host_rows128": {"TFRPN_PIPE_GATHER_ROWS": 128},
+    "device": {"TFRPN_PIPE_GATHER": "device"},
+    "device_rows128": {"TFRPN_PIPE_GATHER": "device", "TFRPN_PIPE_GATHER_ROWS": 128},
+    "matrix": {"TFRPN_NMS_PATH": "matrix"},
+    "matrix_rows128": {"TFRPN_NMS_PATH": "matrix", "TFRPN_PIPE_GATHER_ROWS": 128},
+}
+
+
+@pytest.mark.parametrize("path", list(TWO_PHASE_PATHS))
+@pytest.mark.parametrize("topn", [300, 1000, 6000])
+def test_acquired_tie_scores_collapsed_boxes(cuda_device, path, topn):
+    """Tie-group scores and collapsed regressions through acquired slots.  pre_nms_topn = 300: the rank launch holds
+    every rank (rank_more = 0), and with 128 gathered rows the presorted launch must still send its images to the
+    redo because it could not serve all their ranks.  1000: the rank batch may or may not hold them all.  Six steps:
+    the adaptive gathered-row count grows while images are redone.  B = 6 ranks on 8 x 256, B = 12 on 2 x 512."""
+    if not CO.available():
+        pytest.skip("oracle/_build/librpn_oracle.so not built")
+    B = 12 if path == "host" else 6
+    run_acquired(cuda_device, B, 9, 3, 6, TWO_PHASE_PATHS[path], pre_nms_topn=topn, head=collapsed_head)
+
+
+@pytest.mark.parametrize("rows", [0, 128])
+@pytest.mark.parametrize("topn", [300, 1000, 6000])
+def test_submit_arrays_tie_scores_collapsed_boxes(cuda_device, rows, topn):
+    """the same inputs through submit_arrays on pageable arrays: flagged images are redone when the step is retired"""
+    from tfrpn import HostPipeline
+    if not CO.available():
+        pytest.skip("oracle/_build/librpn_oracle.so not built")
+    hp = dict(O.get_hyper_params("vgg16"))
+    anchors_np = O.generate_anchors(hp)
+    B, depth, P = 6, 3, int(hp["test_nms_topn"])
+    with Env(**({"TFRPN_PIPE_GATHER_ROWS": rows} if rows else {})):
+        pipe = HostPipeline(hp, depth=depth, device=cuda_device, pre_nms_topn=topn)
+    pending = []
+    try:
+        def check(item):
+            t, out, reg, cls = item
+            pipe.wait(t)
+            wb, ws, wv, wk = CO.proposals(reg.reshape(B, -1, 4), cls.reshape(B, -1), anchors_np, hp, topn)
+            assert np.array_equal(out["valid"], wv) and np.array_equal(out["keep_idx"], wk)
+            assert bits_equal(out["scores"], ws) and close(out["boxes"], wb)
+        for i in range(6):
+            reg, cls = collapsed_head(i, B)
+            if len(pending) == depth - 1:
+                check(pending.pop(0))
+            out = dict(boxes=np.full((B, P, 4), np.nan, F32), scores=np.full((B, P), np.nan, F32),
+                       valid=np.full((B,), -7, np.int32), keep_idx=np.full((B, P), -7, np.int32))
+            t, out = pipe.submit_arrays(rpn_reg=reg, rpn_cls=cls, out=out)
+            pending.append((t, out, reg, cls))
         while pending:
             check(pending.pop(0))
     finally:
