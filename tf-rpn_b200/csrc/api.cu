@@ -158,6 +158,8 @@ extern "C" const char* tfrpn_kernel_name(int id) {
         case TFRPN_K_NMS_SWEEP: return "nms_sweep_kernel";
         case TFRPN_K_LOSS: return "rpn_loss_partial_kernel";
         case TFRPN_K_RECALL: return "recall_kernel";
+        case TFRPN_K_NMS_MC_STAGE: return "nms_mc_stage_kernel";
+        case TFRPN_K_NMS_MC_MERGE: return "nms_mc_merge_kernel";
         default: return "?";
     }
 }
@@ -191,6 +193,7 @@ extern "C" int tfrpn_create(tfrpn_handle* out, int device) {
     if (const char* g = getenv("TFRPN_PIPE_EXPAND")) h->opts.pipe_expand = !strcmp(g, "host") ? 1 : (!strcmp(g, "device") ? 2 : 0);
     if (const char* g = getenv("TFRPN_NMS_PATH")) h->opts.nms_lazy = strcmp(g, "matrix") != 0;
     h->opts.nms_rows = env_int("TFRPN_NMS_ROWS", 0);
+    if (const char* g = getenv("TFRPN_NMS_MC_STAGE")) h->opts.nms_mc_stage = !strcmp(g, "column") ? 1 : (!strcmp(g, "rows") ? 2 : 0);
     if (const char* g = getenv("TFRPN_PIPE_GATHER")) h->opts.pipe_gather = !strcmp(g, "host") ? 1 : (!strcmp(g, "device") ? 2 : 0);
     cudaDeviceGetAttribute(&h->sm_count, cudaDevAttrMultiProcessorCount, device);
     // device counter of the loss reduction (losses.cu): zero between calls, the kernel resets it

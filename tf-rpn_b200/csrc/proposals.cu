@@ -25,6 +25,8 @@
 //   nms_mask_kernel, nms_sweep_kernel   matrix NMS over the ranks of a MODE_RANK launch (opt-in, TFRPN_NMS_PATH=matrix)
 //   gather_rows_kernel             candidate rows of a page-locked host tensor -> compact device array (pipeline.cu)
 //   pre_hist / pre_count / pre_scatter_kernel   large-N prefilter (N >= 40 000)
+//   nms_mc_stage_kernel / nms_mc_row_count + nms_mc_row_scatter_kernel, nms_mc_merge_kernel   multi-class combined
+//                                  NMS around proposal_kernel (tfrpn_nms_multiclass)
 // The NMS pair test runs behind a cheap conservative pre-test (nms_maybe / nms_maybe2): see there.
 #include <math.h>
 #include <stdlib.h>
@@ -1447,6 +1449,265 @@ __global__ void __launch_bounds__(SWEEP_THREADS) nms_sweep_kernel(const __grid_c
     if (tid == 0) p.valid[b] = nkept;
 }
 
+// ------------------------------------------------------------------------------------------------
+// Multi-class combined NMS (tfrpn_nms_multiclass): C classes of (B,K,C) scores with shared (q = 1) or
+// class-specific (q = C) boxes.  Three launches:
+//   nms_mc_stage_kernel   one CTA per (image, class): the class's candidates (score > threshold, or all) in
+//                         ASCENDING original index -> compact scores / remap / boxes, the interface of the
+//                         large-N prefilter, so proposal_kernel's composite breaks ties to the lower index
+//                         (column layout: reads column c with stride C).  The same arrays from coalesced score
+//                         rows: nms_mc_row_count_kernel + nms_mc_row_scatter_kernel (row layout, see there)
+//   proposal_kernel       MODE_NMS on the B*C segments (launch_one), keep lists into the workspace
+//   nms_mc_merge_kernel   G CTAs per image: merge the C keep lists by rank, scatter and pad the outputs
+// ------------------------------------------------------------------------------------------------
+constexpr int MC_STAGE_THREADS = 256;
+constexpr int MC_STAGE_ITEMS = 4;      // consecutive positions per thread and sweep step (40 registers: 6 CTAs per SM)
+constexpr int MC_MERGE_THREADS = 512;
+
+struct McStageParams {
+    const float* scores;   // (B,K,C)
+    const float4* boxes;   // (B,K,q)
+    int K, C, q, use_sthr;
+    float sthr;
+    float* cand_scores;    // (B*C, K) per segment, ascending original index
+    int* remap;            // (B*C, K)
+    float4* cand_boxes;    // (B*C, K)
+    int* counts;           // (B*C)
+};
+
+__global__ void __launch_bounds__(MC_STAGE_THREADS) nms_mc_stage_kernel(McStageParams p) {
+    __shared__ unsigned int wtot[MC_STAGE_THREADS / 32];
+    const int seg = blockIdx.x, b = seg / p.C, c = seg - b * p.C;   // the classes of an image run side by side
+    const int tid = threadIdx.x, lane = lane_id(), warp = warp_id();
+    const float* sc = p.scores + (long long)b * p.K * p.C + c;
+    const float4* bx = p.boxes + (long long)b * p.K * p.q + (p.q == 1 ? 0 : c);
+    float* os = p.cand_scores + (long long)seg * p.K;
+    int* orm = p.remap + (long long)seg * p.K;
+    float4* ob = p.cand_boxes + (long long)seg * p.K;
+    unsigned int run = 0;
+    for (int base = 0; base < p.K; base += MC_STAGE_THREADS * MC_STAGE_ITEMS) {
+        const int k0 = base + tid * MC_STAGE_ITEMS;
+        float s[MC_STAGE_ITEMS];
+        unsigned int take = 0;
+#pragma unroll
+        for (int u = 0; u < MC_STAGE_ITEMS; ++u) {
+            s[u] = 0.0f;
+            if (k0 + u < p.K) {
+                s[u] = __ldg(sc + (long long)(k0 + u) * p.C);
+                if (!p.use_sthr || s[u] > p.sthr) take |= 1u << u;   // score_key's rule
+            }
+        }
+        const unsigned int n = __popc(take);
+        const unsigned int incl = (unsigned int)warp_incl_scan((int)n);
+        if (lane == 31) wtot[warp] = incl;
+        __syncthreads();
+        unsigned int woff = 0, tot = 0;
+#pragma unroll
+        for (int w = 0; w < MC_STAGE_THREADS / 32; ++w) {
+            const unsigned int t = wtot[w];
+            woff += w < warp ? t : 0u;
+            tot += t;
+        }
+        __syncthreads();                                // wtot is rewritten by the next step
+        unsigned int o = run + woff + incl - n;
+#pragma unroll
+        for (int u = 0; u < MC_STAGE_ITEMS; ++u) {
+            if ((take >> u) & 1u) {
+                const int k = k0 + u;
+                os[o] = s[u];
+                orm[o] = k;
+                ob[o] = ldg_f4(bx + (long long)k * p.q);
+                ++o;
+            }
+        }
+        run += tot;
+    }
+    if (tid == 0) p.counts[seg] = (int)run;
+}
+
+// Row layout of the staging: grid (slices, B) over coalesced (K, C) score rows, like pre_count / pre_scatter_kernel.
+// Warp w of slice s owns rows [r_lo, r_hi) (flat elements [r_lo * C, r_hi * C), read 32 consecutive at a time).
+// count: candidates per (image, slice, warp, class) -> row_cnt; scatter: each CTA turns the counts of the
+// (slice, warp) pairs before its own into per-warp, per-class offsets (the last slice also writes counts[]), then
+// every warp walks its range in order; lanes with the same class rank themselves with __match_any_sync.
+constexpr int MC_ROW_THREADS = 256;
+constexpr int MC_ROW_WARPS = MC_ROW_THREADS / 32;
+constexpr int MC_ROW_MAX_C = 1024;     // the per-warp, per-class table lives in shared memory (32 KB)
+struct McRowParams {
+    McStageParams g;
+    int slices, slice_rows;
+    int* row_cnt;          // (B, slices, MC_ROW_WARPS, C)
+};
+__device__ __forceinline__ void mc_row_range(const McRowParams& p, int& lo, int& hi) {
+    const int slo = blockIdx.x * p.slice_rows, shi = min(p.g.K, slo + p.slice_rows);
+    const int sub = (p.slice_rows + MC_ROW_WARPS - 1) / MC_ROW_WARPS;
+    const int rlo = min(shi, slo + warp_id() * sub), rhi = min(shi, rlo + sub);
+    lo = rlo * p.g.C;
+    hi = rhi * p.g.C;
+}
+__global__ void __launch_bounds__(MC_ROW_THREADS) nms_mc_row_count_kernel(McRowParams p) {
+    extern __shared__ unsigned int wc[];   // [MC_ROW_WARPS][C]
+    const int b = blockIdx.y, lane = lane_id(), warp = warp_id(), Cn = p.g.C;
+    unsigned int* mine = wc + warp * Cn;
+    for (int c = lane; c < Cn; c += 32) mine[c] = 0u;
+    __syncwarp();
+    int lo, hi;
+    mc_row_range(p, lo, hi);
+    const float* sc = p.g.scores + (long long)b * p.g.K * Cn;
+    for (int f = lo + lane; f - lane < hi; f += 32) {
+        const bool in = f < hi;
+        const float s = in ? __ldg(sc + f) : 0.0f;
+        const bool take = in && (!p.g.use_sthr || s > p.g.sthr);
+        const int c = f % Cn;
+        const unsigned m = __match_any_sync(0xffffffffu, take ? c : -1);
+        if (take && lane == __ffs(m) - 1) mine[c] += __popc(m);
+        __syncwarp();
+    }
+    int* out = p.row_cnt + (((long long)b * p.slices + blockIdx.x) * MC_ROW_WARPS + warp) * Cn;
+    for (int c = lane; c < Cn; c += 32) out[c] = (int)mine[c];
+}
+__global__ void __launch_bounds__(MC_ROW_THREADS) nms_mc_row_scatter_kernel(McRowParams p) {
+    extern __shared__ unsigned int off[];   // [MC_ROW_WARPS][C]
+    const int b = blockIdx.y, s = blockIdx.x, lane = lane_id(), warp = warp_id(), Cn = p.g.C;
+    const int* cnt = p.row_cnt + (long long)b * p.slices * MC_ROW_WARPS * Cn;
+    const bool last = s == p.slices - 1;
+    for (int c = threadIdx.x; c < Cn; c += MC_ROW_THREADS) {
+        int run = 0;
+        for (int q = 0; q < s * MC_ROW_WARPS; ++q) run += cnt[(long long)q * Cn + c];
+        for (int w = 0; w < MC_ROW_WARPS; ++w) {
+            off[w * Cn + c] = (unsigned)run;
+            run += cnt[(long long)(s * MC_ROW_WARPS + w) * Cn + c];
+        }
+        if (last) p.g.counts[(long long)b * Cn + c] = run;
+    }
+    __syncthreads();
+    unsigned int* mine = off + warp * Cn;
+    int lo, hi;
+    mc_row_range(p, lo, hi);
+    const float* sc = p.g.scores + (long long)b * p.g.K * Cn;
+    for (int f = lo + lane; f - lane < hi; f += 32) {
+        const bool in = f < hi;
+        const float v = in ? __ldg(sc + f) : 0.0f;
+        const bool take = in && (!p.g.use_sthr || v > p.g.sthr);
+        const int k = f / Cn, c = f - k * Cn;
+        const unsigned m = __match_any_sync(0xffffffffu, take ? c : -1);
+        if (take) {
+            const long long o = ((long long)b * Cn + c) * p.g.K + mine[c] + __popc(m & ((1u << lane) - 1u));
+            p.g.cand_scores[o] = v;
+            p.g.remap[o] = k;
+            p.g.cand_boxes[o] = ldg_f4(p.g.boxes + ((long long)b * p.g.K + k) * p.g.q + (p.g.q == 1 ? 0 : c));
+        }
+        __syncwarp();
+        if (take && lane == __ffs(m) - 1) mine[c] += __popc(m);
+        __syncwarp();
+    }
+}
+
+struct McMergeParams {
+    const float* ks;       // (B*C, P) keep lists of the per-class NMS: scores, boxes, original indices, lengths
+    const float4* kb;
+    const int* ki;
+    const int* kv;
+    int C, P, rows, lmax;  // lmax = min(P, rows): no entry at a list position >= rows can reach an output row
+    int use_smem;          // scratch in dynamic shared memory, else in `gscratch` (per image: scratch_bytes)
+    char* gscratch;
+    long long scratch_bytes;
+    float4* out_boxes;     // (B, rows)
+    float* out_scores;
+    float* out_classes;
+    int* valid;
+    int* keep_idx;
+};
+
+// Merge key: score by VALUE, descending, as a stable torch.sort compares it: +0 == -0, and NaN (either sign) above
+// +inf, every NaN equal.  A keep list is in the kernel's order of orderable(score), which agrees with this key except
+// that -NaN sorts last there: the list read as [+NaN run][-NaN run][rest] (the "virtual" order) is non-increasing.
+__device__ __forceinline__ uint32_t mc_merge_key(float s) {
+    if (isnan(s)) return 0xFFFFFFFFu;
+    return s == 0.0f ? 0x80000000u : orderable(s);
+}
+__device__ __forceinline__ int mc_phys(int v, int m, int a, int bn) {   // virtual -> physical list position
+    return v < a ? v : (v < a + bn ? m - bn + (v - a) : v - bn);
+}
+
+// Grid (B, G): every CTA of an image builds the keys (cheap: <= C * min(P, rows) loads) and ranks every G-th slice of
+// the entries; CTA 0 writes the padding and valid.
+__global__ void __launch_bounds__(MC_MERGE_THREADS) nms_mc_merge_kernel(McMergeParams p) {
+    extern __shared__ float4 smem4[];
+    __shared__ unsigned int s_total;
+    const int b = blockIdx.x, tid = threadIdx.x, lane = lane_id(), warp = warp_id();
+    constexpr int WARPS = MC_MERGE_THREADS / 32;
+    char* base = p.use_smem ? reinterpret_cast<char*>(smem4)
+                            : p.gscratch + ((long long)b * gridDim.y + blockIdx.y) * p.scratch_bytes;
+    int4* meta = reinterpret_cast<int4*>(base);                            // [C] (m, a, bn, L)
+    uint32_t* keys = reinterpret_cast<uint32_t*>(meta + p.C);              // [C][lmax] merge keys, virtual order
+    const long long seg0 = (long long)b * p.C;
+    if (tid == 0) s_total = 0u;
+    __syncthreads();
+    // ---- 1. per list (one warp each): its NaN runs, then its first L = min(m, lmax) merge keys in virtual order
+    unsigned int live = 0;
+    for (int c = warp; c < p.C; c += WARPS) {
+        const long long seg = seg0 + c;
+        const int m = p.kv[seg];
+        const float* s = p.ks + seg * p.P;
+        int a = 0, bn = 0;
+        for (int j = lane; j < m; j += 32) {
+            const float v = s[j];
+            const bool nan = isnan(v);
+            a += (nan && !signbit(v)) ? 1 : 0;
+            bn += (nan && signbit(v)) ? 1 : 0;
+        }
+        a = __reduce_add_sync(0xffffffffu, a);
+        bn = __reduce_add_sync(0xffffffffu, bn);
+        const int L = min(m, p.lmax);
+        if (lane == 0) { meta[c] = make_int4(m, a, bn, L); live += (unsigned int)m; }
+        for (int v = lane; v < L; v += 32) keys[(long long)c * p.lmax + v] = mc_merge_key(s[mc_phys(v, m, a, bn)]);
+    }
+    if (lane == 0 && live) atomicAdd(&s_total, live);
+    __syncthreads();
+    const int nvalid = min((int)s_total, p.rows);
+    // ---- 2. rank of entry (c, v): v + entries of lists c' < c with key >= its key + of lists c' > c with key >
+    //      its key (each list is non-increasing in virtual order: a binary search).  Equal keys go to the lower
+    //      class, then to the earlier position in the class's list.  Entries ranked >= rows are dropped.
+    const long long items = (long long)p.C * p.lmax;
+    for (long long it = (long long)blockIdx.y * MC_MERGE_THREADS + tid; it < items; it += (long long)gridDim.y * MC_MERGE_THREADS) {
+        const int c = (int)(it / p.lmax), v = (int)(it - (long long)c * p.lmax);
+        const int4 mc = meta[c];
+        if (v >= mc.w) continue;
+        const uint32_t key = keys[it];
+        int rank = v;
+        for (int c2 = 0; c2 < p.C && rank < p.rows; ++c2) {
+            if (c2 == c) continue;
+            const uint32_t* kl = keys + (long long)c2 * p.lmax;
+            int lo = 0, hi = meta[c2].w;                // first position whose entry does not precede (c, v)
+            while (lo < hi) {
+                const int mid = (lo + hi) >> 1;
+                const uint32_t k2 = kl[mid];
+                if (c2 < c ? k2 >= key : k2 > key) lo = mid + 1; else hi = mid;
+            }
+            rank += lo;
+        }
+        if (rank < p.rows) {
+            const long long src = (seg0 + c) * p.P + mc_phys(v, mc.x, mc.y, mc.z);
+            const long long o = (long long)b * p.rows + rank;
+            p.out_boxes[o] = p.kb[src];
+            p.out_scores[o] = p.ks[src];
+            p.out_classes[o] = (float)c;
+            if (p.keep_idx) p.keep_idx[o] = p.ki[src];
+        }
+    }
+    // ---- 3. padding rows (TF pads with 0; keep_idx with -1)
+    if (blockIdx.y != 0) return;
+    for (int r = nvalid + tid; r < p.rows; r += MC_MERGE_THREADS) {
+        const long long o = (long long)b * p.rows + r;
+        p.out_boxes[o] = make_float4(0.f, 0.f, 0.f, 0.f);
+        p.out_scores[o] = 0.0f;
+        p.out_classes[o] = 0.0f;
+        if (p.keep_idx) p.keep_idx[o] = -1;
+    }
+    if (tid == 0) p.valid[b] = nvalid;
+}
+
 static size_t cluster_smem_bytes(int cl, int n_staged, int max_out) {
     max_out = (max_out + 3) & ~3;
     const int T = 1024 / cl;                        // (sort slots per CTA)
@@ -1471,6 +1732,7 @@ int set_attributes_proposals() {
     TFRPN_CHECK_CUDA(cudaFuncSetAttribute(proposal_cluster_kernel<4, 512>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
     TFRPN_CHECK_CUDA(cudaFuncSetAttribute(proposal_cluster_kernel<8, 256>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
     TFRPN_CHECK_CUDA(cudaFuncSetAttribute(proposal_cluster_kernel<8, 512>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
+    TFRPN_CHECK_CUDA(cudaFuncSetAttribute(nms_mc_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
     return 0;
 }
 
@@ -2165,6 +2427,145 @@ extern "C" int tfrpn_proposals_anchor_cfg(tfrpn_handle h, const float* rpn_reg, 
         return fail(TFRPN_ERR_UNSUPPORTED, "proposals_anchor_cfg: N = %lld takes the prefilter path, which reads an anchor tensor; "
                                            "call tfrpn_anchors + tfrpn_proposals", N);
     return launch_one(h, p, B, st);
+}
+
+// ---- multi-class combined NMS (kernels: see nms_mc_stage_kernel) -------------------------------------------------
+namespace tfrpn {
+struct McLayout {
+    int rows, lmax;
+    int G;               // merge CTAs per image
+    int row_layout, slices, slice_rows;   // staging: row layout (count + scatter) and its slices, or the column layout
+    long long scratch;   // merge scratch per CTA: C * 16 + C * lmax * 4 bytes, rounded up to 16
+    size_t cand_scores, remap, cand_boxes, counts, ks, ki, kb, kv, gscratch, row_cnt, total;   // byte offsets, total size
+};
+// Staging layout: TFRPN_NMS_MC_STAGE=column|rows forces one (A/B switch).  Otherwise the column layout once its B*C
+// CTAs fill the 148 SMs, the row layout below that (measured, DESIGN.md section 4: column 62 against 95 us at SSD-VOC,
+// B*C = 640; rows 60 against 150 us at 4 x 100000 x 4, B*C = 16).  The row layout needs C <= MC_ROW_MAX_C.
+static bool mc_rows_apply(int mode, int B, int K, int C) {
+    if (C > MC_ROW_MAX_C || (long long)K * C > 0x7FFFFFFFLL || mode == 1) return false;
+    return mode == 2 || (long long)B * C < 148;
+}
+static void mc_layout(int B, int K, int C, const tfrpn_nms_cfg* cfg, McLayout* L, int stage_mode = 0) {
+    const int P = cfg->max_output_size_per_class;
+    L->rows = cfg->pad_per_class ? (int)std::min((long long)cfg->max_total_size, (long long)P * C) : cfg->max_total_size;
+    L->lmax = min(P, L->rows);
+    L->scratch = ((long long)C * 16 + (long long)C * L->lmax * 4 + 15) & ~15LL;
+    // ~2 CTAs per SM over the batch, no more than there are slices of MC_MERGE_THREADS entries
+    const long long slices = ((long long)C * L->lmax + MC_MERGE_THREADS - 1) / MC_MERGE_THREADS;
+    L->G = (int)std::max(1LL, std::min({slices, (long long)(296 + B - 1) / B, 64LL}));
+    const size_t S = (size_t)B * C;
+    size_t o = 0;
+    L->cand_scores = o; o += align256(S * K * 4);
+    L->remap = o;       o += align256(S * K * 4);
+    L->cand_boxes = o;  o += align256(S * K * 16);
+    L->counts = o;      o += align256(S * 4);
+    L->ks = o;          o += align256(S * P * 4);
+    L->ki = o;          o += align256(S * P * 4);
+    L->kb = o;          o += align256(S * P * 16);
+    L->kv = o;          o += align256(S * 4);
+    L->gscratch = o;    o += align256((size_t)B * L->G * L->scratch);
+    // row layout: ~4 CTAs per SM over the batch, at least 256 rows per slice
+    L->row_layout = mc_rows_apply(stage_mode, B, K, C) ? 1 : 0;
+    L->slices = std::max(1, std::min((592 + B - 1) / B, (K + 255) / 256));
+    L->slice_rows = (K + L->slices - 1) / L->slices;
+    L->row_cnt = o;     o += align256((size_t)B * L->slices * MC_ROW_WARPS * C * 4);   // (counted in every mode)
+    L->total = o + 256;
+}
+static int mc_check_sizes(const char* fn, int B, int K, int C, const tfrpn_nms_cfg* cfg) {
+    if (!cfg) return fail(TFRPN_ERR_BAD_ARG, "%s: null cfg", fn);
+    if (B <= 0 || K <= 0 || C < 1) return fail(TFRPN_ERR_BAD_ARG, "%s: B=%d, K=%d, C=%d must be > 0", fn, B, K, C);
+    if ((long long)B * C > 0x7FFFFFFFLL) return fail(TFRPN_ERR_BAD_ARG, "%s: B * C = %lld segments", fn, (long long)B * C);
+    if (cfg->max_output_size_per_class <= 0 || cfg->max_total_size <= 0)
+        return fail(TFRPN_ERR_BAD_ARG, "%s: max_output_size_per_class and max_total_size must be > 0", fn);
+    if (cfg->pre_nms_topn < 0) return fail(TFRPN_ERR_BAD_ARG, "%s: pre_nms_topn must be >= 0", fn);
+    return 0;
+}
+}  // namespace tfrpn
+
+extern "C" size_t tfrpn_nms_multiclass_workspace_bytes(int B, int K, int C, const tfrpn_nms_cfg* cfg) {
+    if (!cfg || B <= 0 || K <= 0 || C < 1 || cfg->max_output_size_per_class <= 0 || cfg->max_total_size <= 0) return 0;
+    McLayout L;
+    mc_layout(B, K, C, cfg, &L);
+    return L.total;
+}
+
+extern "C" int tfrpn_reserve_nms_multiclass(tfrpn_handle h, int B, int K, int C, const tfrpn_nms_cfg* cfg) {
+    if (!h) return fail(TFRPN_ERR_BAD_ARG, "reserve_nms_multiclass: null handle");
+    if (int rc = mc_check_sizes("reserve_nms_multiclass", B, K, C, cfg)) return rc;
+    TFRPN_ENTER(h);
+    char* ws;
+    return ensure_workspace_prop(h, tfrpn_nms_multiclass_workspace_bytes(B, K, C, cfg), nullptr, &ws);
+}
+
+extern "C" int tfrpn_nms_multiclass(tfrpn_handle h, const float* boxes, int q, const float* scores, int B, int K, int C,
+                                    const tfrpn_nms_cfg* cfg, float* out_boxes, float* out_scores, float* out_classes,
+                                    int32_t* valid, int32_t* keep_idx_or_null, tfrpn_stream s) {
+    if (!boxes || !scores || !cfg || !out_boxes || !out_scores || !out_classes || !valid)
+        return fail(TFRPN_ERR_BAD_ARG, "nms_multiclass: null pointer");
+    if (int rc = mc_check_sizes("nms_multiclass", B, K, C, cfg)) return rc;
+    if (q != 1 && q != C) return fail(TFRPN_ERR_BAD_ARG, "nms_multiclass: q = %d must be 1 or C = %d", q, C);
+    if (!aligned16(boxes) || !aligned16(out_boxes))
+        return fail(TFRPN_ERR_MISALIGNED, "nms_multiclass: boxes must be 16-byte aligned");
+    if (!h) return fail(TFRPN_ERR_BAD_ARG, "nms_multiclass: null handle");
+    TFRPN_ENTER(h);
+    TFRPN_CHECK_ON_DEVICE(h, boxes, "nms_multiclass: boxes");
+    cudaStream_t st = as_stream(s);
+    const int S = B * C, P = cfg->max_output_size_per_class;
+    {   // the per-class kernel's shared-memory carve bounds max_output_size_per_class, as in tfrpn_nms
+        int cl = 0, threads = 1024;
+        pick_cluster(h, S, cl, threads);
+        const size_t smem = cl ? cluster_smem_bytes(cl, 0, P) : prop_smem_bytes(0, P);
+        if (smem > PROP_SMEM_LIMIT)
+            return fail(TFRPN_ERR_UNSUPPORTED, "NMS: %d output rows need %zu B of shared memory (> %zu)", P, smem,
+                        PROP_SMEM_LIMIT);
+    }
+    McLayout L;
+    mc_layout(B, K, C, cfg, &L, h->opts.nms_mc_stage);
+    char* ws = nullptr;
+    if (int rc = ensure_workspace_prop(h, L.total, st, &ws)) return rc;
+
+    McStageParams g = {};
+    g.scores = scores; g.boxes = reinterpret_cast<const float4*>(boxes); g.K = K; g.C = C; g.q = q;
+    g.use_sthr = !(cfg->score_threshold == -INFINITY); g.sthr = cfg->score_threshold;
+    g.cand_scores = reinterpret_cast<float*>(ws + L.cand_scores); g.remap = reinterpret_cast<int*>(ws + L.remap);
+    g.cand_boxes = reinterpret_cast<float4*>(ws + L.cand_boxes); g.counts = reinterpret_cast<int*>(ws + L.counts);
+    prof_begin(h, TFRPN_K_NMS_MC_STAGE, st);
+    if (L.row_layout) {
+        McRowParams r = {};
+        r.g = g; r.slices = L.slices; r.slice_rows = L.slice_rows; r.row_cnt = reinterpret_cast<int*>(ws + L.row_cnt);
+        const size_t smem = (size_t)MC_ROW_WARPS * C * 4;
+        nms_mc_row_count_kernel<<<dim3(L.slices, B), MC_ROW_THREADS, smem, st>>>(r);
+        TFRPN_AFTER_LAUNCH("nms_mc_row_count_kernel");
+        nms_mc_row_scatter_kernel<<<dim3(L.slices, B), MC_ROW_THREADS, smem, st>>>(r);
+    } else {
+        nms_mc_stage_kernel<<<S, MC_STAGE_THREADS, 0, st>>>(g);
+    }
+    prof_end(h, st);
+    TFRPN_AFTER_LAUNCH("nms_mc_stage_kernel");
+
+    PropParams p = {};
+    p.mode = MODE_NMS; p.N = K; p.k = cfg->pre_nms_topn > 0 ? min(K, cfg->pre_nms_topn) : K;
+    p.scores = g.cand_scores; p.counts = g.counts; p.remap = g.remap;
+    p.use_sthr = g.use_sthr; p.score_threshold = g.sthr;
+    p.boxes = g.cand_boxes; p.box_stride = K;
+    p.rows = P; p.max_out = P;
+    p.iou_thr = make_threshold(cfg->iou_threshold); p.clip_out = cfg->clip_boxes;
+    p.out_boxes = reinterpret_cast<float4*>(ws + L.kb); p.out_scores = reinterpret_cast<float*>(ws + L.ks);
+    p.out_classes = nullptr; p.valid = reinterpret_cast<int*>(ws + L.kv); p.keep_idx = reinterpret_cast<int*>(ws + L.ki);
+    if (int rc = launch_one(h, p, S, st)) return rc;
+
+    McMergeParams m = {};
+    m.ks = p.out_scores; m.kb = p.out_boxes; m.ki = p.keep_idx; m.kv = p.valid;
+    m.C = C; m.P = P; m.rows = L.rows; m.lmax = L.lmax;
+    m.use_smem = (size_t)L.scratch <= PROP_SMEM_LIMIT ? 1 : 0;
+    m.gscratch = ws + L.gscratch; m.scratch_bytes = L.scratch;
+    m.out_boxes = reinterpret_cast<float4*>(out_boxes); m.out_scores = out_scores; m.out_classes = out_classes;
+    m.valid = valid; m.keep_idx = keep_idx_or_null;
+    prof_begin(h, TFRPN_K_NMS_MC_MERGE, st);
+    nms_mc_merge_kernel<<<dim3(B, L.G), MC_MERGE_THREADS, m.use_smem ? (size_t)L.scratch : 0, st>>>(m);
+    prof_end(h, st);
+    TFRPN_AFTER_LAUNCH("nms_mc_merge_kernel");
+    return 0;
 }
 
 #ifdef TFRPN_PHASE_TIMING

@@ -55,7 +55,7 @@ class StepBuffers(C.Structure):
 
 P = C.c_void_p
 I = C.c_int
-KERNEL_IDS = 9   # TFRPN_K_COUNT of include/tfrpn.h
+KERNEL_IDS = 11  # TFRPN_K_COUNT of include/tfrpn.h
 # name -> (restype, argtypes); must list every symbol include/tfrpn.h declares
 PROTOTYPES = {
     "tfrpn_version": (I, []),
@@ -106,6 +106,9 @@ PROTOTYPES = {
     "tfrpn_host_alloc": (I, [C.POINTER(P), C.c_size_t]),
     "tfrpn_host_free": (I, [P]),
     "tfrpn_proposal_recall": (I, [P, P, P, P, P, I, I, I, C.POINTER(RecallCfg), P, P, P]),
+    "tfrpn_nms_multiclass": (I, [P, P, I, P, I, I, I, C.POINTER(NmsCfg), P, P, P, P, P, P]),
+    "tfrpn_nms_multiclass_workspace_bytes": (C.c_size_t, [I, I, I, C.POINTER(NmsCfg)]),
+    "tfrpn_reserve_nms_multiclass": (I, [P, I, I, I, C.POINTER(NmsCfg)]),
 }
 
 _lib = None

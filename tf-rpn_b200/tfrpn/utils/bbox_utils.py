@@ -104,56 +104,38 @@ def non_max_suppression(pred_bboxes, pred_labels, **kwargs):
 
 
 def _multi_class_nms(boxes, scores, kwargs, o):
-    """tf.image.combined_non_max_suppression with C > 1 classes (the reference's wrapper allows ``total_labels`` > 1,
-    utils/bbox_utils.py:53-55; the RPN itself has one).  Not a hot path of the reference: every (image, class) pair
-    runs through the one-class kernel as an image of its own, and the per-class keep lists are merged by score with
-    torch (stable sort: equal scores -> lower class id first, then the class's own order -- TF leaves ties to an
-    unstable std::sort)."""
+    """tf.image.combined_non_max_suppression with C > 1 classes or q = C boxes per entry (the reference's wrapper allows
+    ``total_labels`` > 1, utils/bbox_utils.py:53-55; the RPN itself has one), in one tfrpn_nms_multiclass call: per
+    (image, class) the one-class NMS, then the merge of the C keep lists by score (equal scores -> lower class id first,
+    then the class's own order -- TF leaves ties to an unstable std::sort)."""
     B, K, Cn = scores.shape
     q = boxes.shape[2]
     if q not in (1, Cn):
         raise ValueError("pred_bboxes must be (B,K,1,4) or (B,K,C,4) for pred_labels (B,K,C); got q = %d, C = %d" % (q, Cn))
-    per_class, total = int(kwargs["max_output_size_per_class"]), int(kwargs["max_total_size"])
-    pad = bool(kwargs.get("pad_per_class", False))
-    rows = min(total, per_class * Cn) if pad else total
-    dev = boxes.device
-    sc_t = scores.permute(0, 2, 1).contiguous().reshape(B * Cn, K)
-    bx_t = (boxes.expand(B, K, Cn, 4) if q == 1 else boxes).permute(0, 2, 1, 3).contiguous().reshape(B * Cn, K, 4)
-    cfg = _lib.NmsCfg(per_class, per_class, float(kwargs.get("iou_threshold", 0.5)),
-                      float(kwargs.get("score_threshold", float("-inf"))), 0, int(bool(kwargs.get("clip_boxes", True))),
+    cfg = _lib.NmsCfg(int(kwargs["max_output_size_per_class"]), int(kwargs["max_total_size"]),
+                      float(kwargs.get("iou_threshold", 0.5)), float(kwargs.get("score_threshold", float("-inf"))),
+                      int(bool(kwargs.get("pad_per_class", False))), int(bool(kwargs.get("clip_boxes", True))),
                       int(kwargs.get("pre_nms_topn") or 0))
-    nb = torch.empty((B * Cn, per_class, 4), dtype=F32, device=dev)
-    ns = torch.empty((B * Cn, per_class), dtype=F32, device=dev)
-    nc = torch.empty((B * Cn, per_class), dtype=F32, device=dev)
-    nv = torch.empty((B * Cn,), dtype=torch.int32, device=dev)
-    ni = torch.empty((B * Cn, per_class), dtype=torch.int32, device=dev)
-    _lib.check(_lib.load().tfrpn_nms(_lib.handle(dev.index), ptr(bx_t), ptr(sc_t), B * Cn, K, C.byref(cfg),
-                                     ptr(nb), ptr(ns), ptr(nc), ptr(nv), ptr(ni), stream_ptr(dev)))
-    # merge the C keep lists of an image: flat slot = class * per_class + position, so a stable descending sort
-    # breaks ties by class, then by position
-    slot = torch.arange(per_class, device=dev)
-    live = slot[None, :] < nv[:, None]                                         # (B*C, per_class)
-    key = torch.where(live, ns, torch.full_like(ns, float("-inf"))).reshape(B, Cn * per_class)
-    order = torch.sort(key, dim=1, descending=True, stable=True).indices       # (B, C*per_class)
-    n_live = live.reshape(B, -1).sum(dim=1)
-    take = min(rows, Cn * per_class)
-    order = order[:, :take]
-    valid = torch.clamp(n_live, max=min(rows, total)).to(torch.int32)
-    keep = torch.arange(take, device=dev)[None, :] < valid[:, None]            # (B, take)
-    ob = torch.zeros((B, rows, 4), dtype=F32, device=dev)
-    os_ = torch.zeros((B, rows), dtype=F32, device=dev)
-    oc = torch.zeros((B, rows), dtype=F32, device=dev)
-    oi = torch.full((B, rows), -1, dtype=torch.int32, device=dev)
-    gb = torch.gather(nb.reshape(B, Cn * per_class, 4), 1, order[..., None].expand(-1, -1, 4))
-    gs = torch.gather(ns.reshape(B, Cn * per_class), 1, order)
-    gi = torch.gather(ni.reshape(B, Cn * per_class), 1, order)
-    ob[:, :take] = torch.where(keep[..., None], gb, torch.zeros_like(gb))
-    os_[:, :take] = torch.where(keep, gs, torch.zeros_like(gs))
-    oc[:, :take] = torch.where(keep, (order // per_class).to(F32), torch.zeros_like(gs))
-    oi[:, :take] = torch.where(keep, gi, torch.full_like(gi, -1))
-    res = NmsOutput(*(from_device(t, o) for t in (ob, os_, oc, valid)))
+    if cfg.max_output_size_per_class <= 0 or cfg.max_total_size <= 0:
+        raise ValueError("max_output_size_per_class and max_total_size must be > 0")
+    rows = min(cfg.max_total_size, cfg.max_output_size_per_class * Cn) if cfg.pad_per_class else cfg.max_total_size
+    dev = boxes.device
+    run = B > 0 and K > 0 and Cn > 0   # the kernels write every output; without boxes or classes every row is padding
+    alloc = torch.empty if run else torch.zeros
+    nb = alloc((B, rows, 4), dtype=F32, device=dev)
+    ns = alloc((B, rows), dtype=F32, device=dev)
+    nc = alloc((B, rows), dtype=F32, device=dev)
+    nv = alloc((B,), dtype=torch.int32, device=dev)
+    ni = None
     if kwargs.get("return_indices"):
-        return tuple(res) + (from_device(oi, o),)
+        ni = torch.empty((B, rows), dtype=torch.int32, device=dev) if run else torch.full((B, rows), -1, dtype=torch.int32, device=dev)
+    if run:
+        _lib.check(_lib.load().tfrpn_nms_multiclass(_lib.handle(dev.index), ptr(boxes), q, ptr(scores), B, K, Cn,
+                                                    C.byref(cfg), ptr(nb), ptr(ns), ptr(nc), ptr(nv), ptr(ni),
+                                                    stream_ptr(dev)))
+    res = NmsOutput(*(from_device(t, o) for t in (nb, ns, nc, nv)))
+    if ni is not None:
+        return tuple(res) + (from_device(ni, o),)
     return res
 
 
