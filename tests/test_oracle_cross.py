@@ -5,6 +5,7 @@ import pytest
 
 from oracle import c_oracle as CO
 from oracle import rpn_oracle as O
+from oracle import target_layouts as TL
 
 F32 = np.float32
 pytestmark = pytest.mark.skipif(not CO.available(), reason="C oracle not built (make -C oracle)")
@@ -40,6 +41,36 @@ def test_targets_numpy_vs_c(bb, B, G):
     assert np.array_equal(cdbg["pos_pre"].astype(bool), dbg["pos_pre"])
     assert np.array_equal(cdbg["neg_pre"].astype(bool), dbg["neg_pre"])
     assert np.array_equal(cd != 0, d != 0) and close(cd, d)
+
+
+@pytest.mark.parametrize("name", TL.FALLBACK_LAYOUTS)
+def test_targets_numpy_vs_c_fallback_layouts(name):
+    """Pixel coordinates, tiny coordinates, flipped boxes, NaN / inf, zero-area anchors, NaN columns
+    (oracle/target_layouts.py).  The NumPy oracle takes np.maximum / np.minimum (NaN-propagating), the C oracle
+    fmaxf / fminf (NaN-ignoring): a NaN coordinate still gives a NaN area, hence a NaN union and IoU, on both
+    sides, and inf - inf inside the intersection only arises with an infinite extent, whose area is NaN too.
+    So the two agree on every output, bit for bit, except one: max_iou where an anchor's best IoU is a zero of
+    both signs (a flipped GT box of negative area gives -0).  The C oracle keeps the first maximal value (its
+    `v > best` scan), as the kernel does; NumPy's max reduction may return the other zero.  The values are equal,
+    so no threshold sees the difference."""
+    anchors, gtb, gtl = TL.fallback_layout(name)
+    B, N = gtl.shape[0], anchors.shape[0]
+    hp = dict(O.get_hyper_params("vgg16"), feature_map_shape=(1, N))
+    hp["anchor_count"] = 1
+    with np.errstate(invalid="ignore", over="ignore"):
+        d, l, dbg = O.calculate_rpn_actual_outputs(anchors, gtb, gtl, hp, seed=3, offset=5, image_offset=1,
+                                                   return_debug=True)
+    cd, cl, cdbg = CO.rpn_targets(anchors, gtb, gtl, hp, seed=3, offset=5, image_offset=1, debug=True)
+    assert np.array_equal(bits(cl), bits(l.reshape(B, -1)))
+    assert np.array_equal(cdbg["argmax_row"], dbg["argmax_row"]) and np.array_equal(cdbg["argmax_col"], dbg["argmax_col"])
+    assert np.array_equal(cdbg["max_iou"], dbg["max_iou"])
+    zero = cdbg["max_iou"] == 0
+    assert np.array_equal(bits(cdbg["max_iou"])[~zero], bits(dbg["max_iou"])[~zero])
+    assert np.array_equal(cdbg["pos_pre"].astype(bool), dbg["pos_pre"])
+    assert np.array_equal(cdbg["neg_pre"].astype(bool), dbg["neg_pre"])
+    assert np.array_equal(np.isnan(cd), np.isnan(d))
+    fin = ~np.isnan(d)
+    assert np.array_equal(cd[fin] != 0, d[fin] != 0) and close(cd[fin], d[fin])
 
 
 def test_select_topk_proposals_numpy_vs_c():
