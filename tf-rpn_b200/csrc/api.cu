@@ -160,6 +160,8 @@ extern "C" const char* tfrpn_kernel_name(int id) {
         case TFRPN_K_RECALL: return "recall_kernel";
         case TFRPN_K_NMS_MC_STAGE: return "nms_mc_stage_kernel";
         case TFRPN_K_NMS_MC_MERGE: return "nms_mc_merge_kernel";
+        case TFRPN_K_MAP_MATCH: return "map_match_kernel";
+        case TFRPN_K_MAP_AP: return "map_ap_kernel";
         default: return "?";
     }
 }

@@ -9,6 +9,6 @@ from . import _lib  # noqa: F401
 from .utils import bbox_utils, data_utils, train_utils  # noqa: F401
 from .proposals import generate_proposals, predict_top_boxes  # noqa: F401
 from .pipeline import HostPipeline, prefetching_rpn_generator  # noqa: F401
-from .evaluation import ProposalRecall, proposal_recall  # noqa: F401
+from .evaluation import DetectionMAP, ProposalRecall, detection_map, proposal_recall  # noqa: F401
 
 __version__ = "0.1.0"

@@ -48,6 +48,16 @@ class RecallCfg(C.Structure):
                 ("limits", C.c_int32 * 8), ("matching", C.c_int32), ("reserved", C.c_int32)]
 
 
+class MapCfg(C.Structure):
+    _fields_ = [("protocol", C.c_int32), ("num_classes", C.c_int32), ("n_thresholds", C.c_int32),
+                ("thresholds", C.c_float * 16), ("max_dets", C.c_int32), ("reserved", C.c_int32)]
+
+
+class MapState(C.Structure):
+    _fields_ = [("records", C.c_void_p), ("capacity", C.c_int64), ("cursor", C.c_void_p), ("n_gt", C.c_void_p),
+                ("overflow", C.c_void_p)]
+
+
 class StepBuffers(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("gt_boxes", "gt_labels", "rpn_reg", "rpn_cls", "deltas", "labels",
                                           "out_boxes", "out_scores", "valid", "keep_idx")]
@@ -55,7 +65,7 @@ class StepBuffers(C.Structure):
 
 P = C.c_void_p
 I = C.c_int
-KERNEL_IDS = 11  # TFRPN_K_COUNT of include/tfrpn.h
+KERNEL_IDS = 13  # TFRPN_K_COUNT of include/tfrpn.h
 # name -> (restype, argtypes); must list every symbol include/tfrpn.h declares
 PROTOTYPES = {
     "tfrpn_version": (I, []),
@@ -109,6 +119,9 @@ PROTOTYPES = {
     "tfrpn_nms_multiclass": (I, [P, P, I, P, I, I, I, C.POINTER(NmsCfg), P, P, P, P, P, P]),
     "tfrpn_nms_multiclass_workspace_bytes": (C.c_size_t, [I, I, I, C.POINTER(NmsCfg)]),
     "tfrpn_reserve_nms_multiclass": (I, [P, I, I, I, C.POINTER(NmsCfg)]),
+    "tfrpn_map_update": (I, [P, P, P, P, P, P, P, P, I, I, I, C.POINTER(MapCfg), C.POINTER(MapState), P]),
+    "tfrpn_map_compute": (I, [P, C.POINTER(MapCfg), C.POINTER(MapState), P, P, P]),
+    "tfrpn_map_workspace_bytes": (C.c_size_t, [C.c_int64, I]),
 }
 
 _lib = None
