@@ -186,6 +186,7 @@ extern "C" int tfrpn_create(tfrpn_handle* out, int device) {
     h->opts.pipe_dense = getenv("TFRPN_PIPE_DENSE") != nullptr;
     h->opts.pipe_chunks = env_int("TFRPN_PIPE_CHUNKS", 0);
     h->opts.prop_cluster = env_int("TFRPN_PROP_CLUSTER", -1);
+    h->opts.prop_threads = env_int("TFRPN_PROP_THREADS", 0);
     h->opts.pipe_dense_in = getenv("TFRPN_PIPE_DENSE_IN") != nullptr;
     h->opts.pipe_trace = getenv("TFRPN_PIPE_TRACE") != nullptr;
     h->opts.pipe_gather_rows = env_int("TFRPN_PIPE_GATHER_ROWS", 0);

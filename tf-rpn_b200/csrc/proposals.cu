@@ -19,7 +19,8 @@
 //   In the fused mode boxes are decoded (+clipped) on the fly, for the examined candidates only.
 //
 // Kernels of this file:
-//   proposal_kernel                one 1024-thread CTA per image (the default above 8 images per launch)
+//   proposal_kernel<T>             one CTA of T = 512 (two per SM) or 1024 threads per image (the default above 8
+//                                  images per launch; launch_one picks T)
 //   proposal_cluster_kernel<CL,T>  the same algorithm on a thread-block cluster per image (<= 8 images per launch;
 //                                  also MODE_RANK / presorted launches of the host pipeline's two-phase transfer)
 //   nms_mask_kernel, nms_sweep_kernel   matrix NMS over the ranks of a MODE_RANK launch (opt-in, TFRPN_NMS_PATH=matrix)
@@ -42,11 +43,8 @@ namespace cg = cooperative_groups;
 
 namespace tfrpn {
 
-constexpr int PR_THREADS = 1024;
-constexpr int PR_WARPS = PR_THREADS / 32;
-constexpr int BATCH = PR_THREADS;   // ranks sorted per batch: one composite per thread
+constexpr int BATCH = 1024;         // ranks sorted per batch: BATCH / T composites per thread of proposal_kernel<T>
 constexpr int NMS_CHUNK = 128;
-constexpr int NMS_PARTS = PR_THREADS / NMS_CHUNK;  // 8
 
 enum { MODE_TOPK = 0, MODE_NMS = 1, MODE_PROPOSALS = 2, MODE_RANK = 3 };
 
@@ -128,7 +126,7 @@ constexpr int SEL_LIST = 2 * BATCH;        // candidate-list capacity: the sort 
 constexpr int SEG_MAX = 32;                // longest counting-sort bin ordered by comparisons; longer -> bitonic network
 
 struct PropShared {
-    unsigned int wtot[PR_WARPS], wmax[PR_WARPS];
+    unsigned int wtot[32], wmax[32];
     unsigned int digit, excl, bin_count;
     unsigned int count;      // entries above the score threshold
     unsigned int lcount;     // candidate-list cursor
@@ -151,24 +149,53 @@ __device__ __forceinline__ unsigned long long make_comp(uint32_t key, int i) {
     return ((unsigned long long)key << 32) | (unsigned long long)(0xFFFFFFFFu - (uint32_t)i);
 }
 
-// Block-wide scan of SEL_NB histogram bins from the top: thread t owns bins SEL_NB-1-2t (c0) and SEL_NB-2-2t (c1).
-// excl = entries in the bins above c0, total = all entries, cmax = the fullest bin.  One barrier inside; sh->wtot /
+// Histogram bins of thread t of a T-thread CTA, scanned from the top: PER = SEL_NB / T bins, c[q] = bin
+// SEL_NB-1-PER*t-q.  Four bins are one aligned 16-byte word (read and written as one).
+template <int T>
+__device__ __forceinline__ void own_bins_load(const unsigned int* hist, unsigned (&c)[SEL_NB / T]) {
+    constexpr int PER = SEL_NB / T;
+    const int t = threadIdx.x;
+    if constexpr (PER == 4) {
+        const uint4 v = reinterpret_cast<const uint4*>(hist)[SEL_NB / 4 - 1 - t];
+        c[0] = v.w; c[1] = v.z; c[2] = v.y; c[3] = v.x;
+    } else {
+#pragma unroll
+        for (int q = 0; q < PER; ++q) c[q] = hist[SEL_NB - 1 - PER * t - q];
+    }
+}
+template <int T>
+__device__ __forceinline__ void own_bins_store(unsigned int* hist, const unsigned (&c)[SEL_NB / T]) {
+    constexpr int PER = SEL_NB / T;
+    const int t = threadIdx.x;
+    if constexpr (PER == 4) {
+        reinterpret_cast<uint4*>(hist)[SEL_NB / 4 - 1 - t] = make_uint4(c[3], c[2], c[1], c[0]);
+    } else {
+#pragma unroll
+        for (int q = 0; q < PER; ++q) hist[SEL_NB - 1 - PER * t - q] = c[q];
+    }
+}
+
+// Block-wide scan of SEL_NB histogram bins from the top over the own bins c[] (own_bins_load).
+// excl = entries in the bins above c[0], total = all entries, cmax = the fullest bin.  One barrier inside; sh->wtot /
 // sh->wmax may be rewritten only after another barrier.
-__device__ __forceinline__ void hist_scan_desc(const unsigned int* hist, unsigned& c0, unsigned& c1, unsigned& excl,
+template <int T>
+__device__ __forceinline__ void hist_scan_desc(const unsigned int* hist, unsigned (&c)[SEL_NB / T], unsigned& excl,
                                                unsigned& total, unsigned& cmax, PropShared* sh) {
-    const int t = threadIdx.x, lane = lane_id(), warp = warp_id();
-    c0 = hist[SEL_NB - 1 - 2 * t];
-    c1 = hist[SEL_NB - 2 - 2 * t];
-    const unsigned s = c0 + c1;
+    constexpr int WARPS = T / 32;
+    const int lane = lane_id(), warp = warp_id();
+    own_bins_load<T>(hist, c);
+    unsigned s = 0, m = 0;
+#pragma unroll
+    for (int q = 0; q < SEL_NB / T; ++q) { s += c[q]; m = max(m, c[q]); }
     const unsigned incl = (unsigned)warp_incl_scan((int)s);
-    const unsigned m = __reduce_max_sync(0xffffffffu, max(c0, c1));
+    m = __reduce_max_sync(0xffffffffu, m);
     if (lane == 31) { sh->wtot[warp] = incl; sh->wmax[warp] = m; }
     __syncthreads();
-    const unsigned w = sh->wtot[lane];
+    const unsigned w = lane < WARPS ? sh->wtot[lane] : 0u;
     const unsigned wi = (unsigned)warp_incl_scan((int)w);
     total = __shfl_sync(0xffffffffu, wi, 31);
     excl = __shfl_sync(0xffffffffu, wi - w, warp) + incl - s;
-    cmax = __reduce_max_sync(0xffffffffu, sh->wmax[lane]);
+    cmax = __reduce_max_sync(0xffffffffu, lane < WARPS ? sh->wmax[lane] : 0u);
 }
 
 // TF CombinedNonMaxSuppression IOU on canonicalised boxes ([TF-internal]); c = (ymin,xmin,ymax,xmax).
@@ -233,17 +260,17 @@ __device__ __forceinline__ bool nms_suppresses_filtered(float4 ci, float ai, flo
     return nms_maybe(ci, ai, cj, aj, t.lo_s) && nms_suppresses_fast(ci, ai, cj, aj, t);
 }
 
-// descending bitonic sort of PR_THREADS composites, one per thread; thread t ends with rank t.
+// descending bitonic sort of BATCH composites, one per thread of a BATCH-thread CTA; thread t ends with rank t.
 // Strides < 32 use shuffles; strides >= 32 go through a double-buffered shared array (1 barrier each).
 __device__ __forceinline__ unsigned long long bitonic_sort_desc(unsigned long long v, unsigned long long* buf) {
     const int t = threadIdx.x;
     int flip = 0;
-    for (int k = 2; k <= PR_THREADS; k <<= 1) {
+    for (int k = 2; k <= BATCH; k <<= 1) {
         const bool desc = (t & k) == 0;
         for (int j = k >> 1; j > 0; j >>= 1) {
             unsigned long long pv;
             if (j >= 32) {
-                unsigned long long* bb = buf + flip * PR_THREADS;
+                unsigned long long* bb = buf + flip * BATCH;
                 bb[t] = v;
                 __syncthreads();
                 pv = bb[t ^ j];
@@ -259,7 +286,33 @@ __device__ __forceinline__ unsigned long long bitonic_sort_desc(unsigned long lo
     return v;
 }
 
-__global__ void __launch_bounds__(PR_THREADS, 1) proposal_kernel(PropParams p) {
+// the same network over BATCH composites in shared memory, sorted in place by a CTA of T < BATCH threads: one
+// compare-exchange per pair and step, a barrier after each step
+template <int T>
+__device__ __forceinline__ void bitonic_sort_desc_shared(unsigned long long* buf) {
+    for (int k = 2; k <= BATCH; k <<= 1) {
+        for (int j = k >> 1; j > 0; j >>= 1) {
+            for (int q = threadIdx.x; q < BATCH / 2; q += T) {
+                const int i = ((q & ~(j - 1)) << 1) | (q & (j - 1)), l = i + j;
+                const unsigned long long a = buf[i], c = buf[l];
+                if (((i & k) == 0) == (a < c)) { buf[i] = c; buf[l] = a; }   // descending where bit k of i is 0
+            }
+            __syncthreads();
+        }
+    }
+}
+
+// One CTA of T threads per image (T = 1024 or 512).  The algorithm and every order are the same for both builds; only
+// the mapping of work to threads differs: sweeps stride T, thread t owns SEL_NB / T histogram bins of a scan, holds
+// list entries t + q T and ranks t + q T of the batch, and the kept-list test splits a candidate into T / 128 parts.
+// Two 512-thread CTAs share an SM (64 registers per thread) and fill each other's barrier gaps.
+template <int T>
+__global__ void __launch_bounds__(T, BATCH / T) proposal_kernel(PropParams p) {
+    constexpr int PER_BIN = SEL_NB / T;       // histogram bins per thread in a scan
+    constexpr int PER_LIST = SEL_LIST / T;    // candidate-list entries per thread
+    constexpr int PER_RANK = BATCH / T;       // ranks of a batch per thread
+    constexpr int NMS_PARTS = T / NMS_CHUNK;  // kept-list parts per candidate
+    static_assert((T == 512 || T == 1024) && T >= NMS_CHUNK * 4, "proposal_kernel: 512 or 1024 threads");
     extern __shared__ float4 smem4[];
     __shared__ PropShared sh;
     PH_DECL
@@ -291,21 +344,21 @@ __global__ void __launch_bounds__(PR_THREADS, 1) proposal_kernel(PropParams p) {
 
     // ---- phase 0: stage keys; count entries above the score threshold, the largest key and the first select
     //      histogram (key bits [31:21]) in the same sweep, four loads in flight per thread --------------------
-    hist[2 * tid] = 0u;
-    hist[2 * tid + 1] = 0u;
+#pragma unroll
+    for (int q = 0; q < PER_BIN; ++q) hist[q * T + tid] = 0u;
     if (tid == 0) { sh.count = 0u; sh.kmax = 0u; }
     __syncthreads();
     unsigned int my_valid = 0, my_max = 0;
-    for (int base = 0; base < N; base += 4 * PR_THREADS) {
+    for (int base = 0; base < N; base += 4 * T) {
         float sc[4];
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
-            const int i = base + u * PR_THREADS + tid;
+            const int i = base + u * T + tid;
             sc[u] = i < N ? __ldg(scores + i) : 0.0f;
         }
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
-            const int i = base + u * PR_THREADS + tid;
+            const int i = base + u * T + tid;
             if (i < N) {
                 const uint32_t key = score_key(sc[u], p.use_sthr, p.score_threshold);
                 if (p.staged) skeys[i] = key;
@@ -353,12 +406,12 @@ __global__ void __launch_bounds__(PR_THREADS, 1) proposal_kernel(PropParams p) {
             const unsigned int dmask = (2u << (top - shift)) - 1u;
             const unsigned long long himask = top >= 63 ? 0ull : (~0ull << (top + 1));
             if (nl >= 0) {
-                for (int q = tid; q < nl; q += PR_THREADS) {
+                for (int q = tid; q < nl; q += T) {
                     const unsigned long long c = sortbuf[q];
                     if (((c ^ prefix) & himask) == 0ull) atomicAdd(&hist[(unsigned)(c >> shift) & dmask], 1u);
                 }
             } else if (pass > 0 || have_lo) {           // (the first batch's first histogram comes from phase 0)
-                for (int base = 0; base < N; base += PR_THREADS) {
+                for (int base = 0; base < N; base += T) {
                     const int i = base + tid;
                     unsigned long long c = 0ull;
                     bool in = false;                    // eligible and >= prefix: above the bin, or in it
@@ -380,15 +433,21 @@ __global__ void __launch_bounds__(PR_THREADS, 1) proposal_kernel(PropParams p) {
             }
             __syncthreads();                            // histogram (and list) complete
             if (listing) nl = (int)sh.lcount;
-            unsigned c0, c1, ex0, total, cmax;
-            hist_scan_desc(hist, c0, c1, ex0, total, cmax, &sh);
-            hist[SEL_NB - 1 - 2 * tid] = 0u;             // own bins, for the next histogram (after the barrier below)
-            hist[SEL_NB - 2 - 2 * tid] = 0u;
-            if (ex0 < r && r <= ex0 + c0 + c1) {
-                const bool upper = r <= ex0 + c0;
-                sh.digit = (unsigned)(SEL_NB - 1 - 2 * tid) - (upper ? 0u : 1u);
-                sh.excl = upper ? ex0 : ex0 + c0;
-                sh.bin_count = upper ? c0 : c1;
+            unsigned total;
+            {
+                unsigned c[PER_BIN], ex, cmax;
+                hist_scan_desc<T>(hist, c, ex, total, cmax, &sh);
+                const unsigned zero[PER_BIN] = {};
+                own_bins_store<T>(hist, zero);          // own bins, for the next histogram (after the barrier below)
+#pragma unroll
+                for (int q = 0; q < PER_BIN; ++q) {     // the bin that holds rank r
+                    if (ex < r && r <= ex + c[q]) {
+                        sh.digit = (unsigned)(SEL_NB - 1 - PER_BIN * tid - q);
+                        sh.excl = ex;
+                        sh.bin_count = c[q];
+                    }
+                    ex += c[q];
+                }
             }
             if (tid == 0) sh.lcount = 0u;
             __syncthreads();
@@ -404,9 +463,9 @@ __global__ void __launch_bounds__(PR_THREADS, 1) proposal_kernel(PropParams p) {
             top = shift - 1;                            // (shift == 0 cannot get here: its bins are single composites)
         }
         PH(2);
-        // ---- 2. the batch: up to two list entries per thread (without a list, one compaction sweep makes it) ----
+        // ---- 2. the batch: up to PER_LIST list entries per thread (without a list, one compaction sweep makes it) ----
         if (nl < 0) {
-            for (int base = 0; base < N; base += PR_THREADS) {
+            for (int base = 0; base < N; base += T) {
                 const int i = base + tid;
                 bool take = false;
                 unsigned long long c = 0ull;
@@ -426,68 +485,94 @@ __global__ void __launch_bounds__(PR_THREADS, 1) proposal_kernel(PropParams p) {
             nl = (int)sh.lcount;
         }
         // list entries are eligible and >= tau's bin edge or better; composites of entries are > 0
-        const unsigned long long e0 = tid < nl ? sortbuf[tid] : 0ull;
-        const unsigned long long e1 = tid + BATCH < nl ? sortbuf[tid + BATCH] : 0ull;
-        const bool m0 = e0 != 0ull && e0 >= tau, m1 = e1 != 0ull && e1 >= tau;
+        unsigned long long le[PER_LIST];
+#pragma unroll
+        for (int q = 0; q < PER_LIST; ++q) le[q] = q * T + tid < nl ? sortbuf[q * T + tid] : 0ull;
         PH(3);
         // ---- 3. order the batch: counting sort on the 11 key bits below the common prefix of its key range
         //      [key(tau), upper bound]; a bin's entries find their place by comparing composites within it ---------
         const uint32_t khi = have_lo ? (uint32_t)(lo_tau >> 32) : kmax, kdiff = khi ^ (uint32_t)(tau >> 32);
         const int sshift = kdiff ? max(31 - __clz(kdiff) - (SEL_BITS - 1), 0) : 0;
-        unsigned d0 = 0, d1 = 0, s0 = 0, s1 = 0;
-        if (m0) { d0 = ((uint32_t)(e0 >> 32) >> sshift) & (SEL_NB - 1); s0 = atomicAdd(&hist[d0], 1u); }
-        if (m1) { d1 = ((uint32_t)(e1 >> 32) >> sshift) & (SEL_NB - 1); s1 = atomicAdd(&hist[d1], 1u); }
+        unsigned ds[PER_LIST];                          // (bin << 16) | place in the bin; ~0u: not in the batch
+#pragma unroll
+        for (int q = 0; q < PER_LIST; ++q) {
+            ds[q] = ~0u;
+            if (le[q] != 0ull && le[q] >= tau) {
+                const unsigned d = ((uint32_t)(le[q] >> 32) >> sshift) & (SEL_NB - 1);
+                ds[q] = (d << 16) | atomicAdd(&hist[d], 1u);
+            }
+        }
         __syncthreads();                                // bin counts complete; the list has been read
-        unsigned c0, c1, ex0, total, cmax;
-        hist_scan_desc(hist, c0, c1, ex0, total, cmax, &sh);
-        hist[SEL_NB - 1 - 2 * tid] = (ex0 << 16) | c0;  // (first position, count) of the own bins
-        hist[SEL_NB - 2 - 2 * tid] = ((ex0 + c0) << 16) | c1;
+        unsigned total, cmax;
+        {
+            unsigned c[PER_BIN], ex;
+            hist_scan_desc<T>(hist, c, ex, total, cmax, &sh);
+#pragma unroll
+            for (int q = 0; q < PER_BIN; ++q) { const unsigned n = c[q]; c[q] = (ex << 16) | n; ex += n; }
+            own_bins_store<T>(hist, c);                 // (first position, count) of the own bins
+        }
         __syncthreads();
         const int nb_all = (int)total;                  // entries of this batch, <= BATCH
         unsigned long long* bybin = sortbuf;            // [BATCH] the batch grouped by bin
         unsigned long long* ranked = sortbuf + BATCH;   // [BATCH] the batch in rank order
-        if (m0) bybin[(hist[d0] >> 16) + s0] = e0;
-        if (m1) bybin[(hist[d1] >> 16) + s1] = e1;
+#pragma unroll
+        for (int q = 0; q < PER_LIST; ++q)
+            if (ds[q] != ~0u) bybin[(hist[ds[q] >> 16] >> 16) + (ds[q] & 0xFFFFu)] = le[q];
         __syncthreads();
-        unsigned long long mine;
+        unsigned long long mine[PER_RANK];              // thread t holds ranks t + q T of the batch
         if (cmax <= (unsigned)SEG_MAX) {
-            auto place = [&](unsigned long long e, unsigned d) {
+            auto place = [&](unsigned long long v, unsigned d) {
                 const unsigned hv = hist[d], first = hv >> 16, n = hv & 0xFFFFu;
                 unsigned gt = 0;
-                for (unsigned q = 0; q < n; ++q) gt += bybin[first + q] > e ? 1u : 0u;
-                ranked[first + gt] = e;
+                for (unsigned q = 0; q < n; ++q) gt += bybin[first + q] > v ? 1u : 0u;
+                ranked[first + gt] = v;
             };
-            if (m0) place(e0, d0);
-            if (m1) place(e1, d1);
+#pragma unroll
+            for (int q = 0; q < PER_LIST; ++q)
+                if (ds[q] != ~0u) place(le[q], ds[q] >> 16);
             __syncthreads();
-            mine = tid < nb_all ? ranked[tid] : 0ull;
-        } else {                                        // long bins (tie groups, clustered scores): bitonic network
-            mine = tid < nb_all ? bybin[tid] : 0ull;    // padding sorts last
+#pragma unroll
+            for (int q = 0; q < PER_RANK; ++q) mine[q] = q * T + tid < nb_all ? ranked[q * T + tid] : 0ull;
+        } else if constexpr (T == BATCH) {              // long bins (tie groups, clustered scores): bitonic network
+            mine[0] = tid < nb_all ? bybin[tid] : 0ull; // padding sorts last
             __syncthreads();
-            mine = bitonic_sort_desc(mine, sortbuf);
+            mine[0] = bitonic_sort_desc(mine[0], sortbuf);
+        } else {
+#pragma unroll
+            for (int q = 0; q < PER_RANK; ++q) ranked[q * T + tid] = q * T + tid < nb_all ? bybin[q * T + tid] : 0ull;
+            __syncthreads();
+            bitonic_sort_desc_shared<T>(ranked);
+#pragma unroll
+            for (int q = 0; q < PER_RANK; ++q) mine[q] = ranked[q * T + tid];
         }
-        hist[2 * tid] = 0u;                             // for the next batch: its first histogram follows a barrier
-        hist[2 * tid + 1] = 0u;
-        const int blo = lo;                             // thread t holds rank blo + t
+#pragma unroll
+        for (int q = 0; q < PER_BIN; ++q) hist[q * T + tid] = 0u;   // for the next batch: its first histogram follows a barrier
+        const int blo = lo;                             // thread t holds ranks blo + t + q T
         const int nb = min(nb_all, K - lo);             // entries of this batch that may be consumed
         lo += nb_all;
         lo_tau = tau;
         have_lo = true;
         PH(4);
-        const uint32_t my_i = 0xFFFFFFFFu - (uint32_t)(mine & 0xFFFFFFFFull);
+        uint32_t my_i[PER_RANK];
+#pragma unroll
+        for (int q = 0; q < PER_RANK; ++q) my_i[q] = 0xFFFFFFFFu - (uint32_t)(mine[q] & 0xFFFFFFFFull);
 
         // ---- 4a. top-k outputs (predictor.py:58-60) -------------------------------------------
         if (p.mode == MODE_TOPK) {
-            if (tid < nb) {
-                const long long o = (long long)b * p.k + blo + tid;
-                p.values[o] = scores[my_i];
-                p.indices[o] = remap ? remap[my_i] : (int)my_i;
+#pragma unroll
+            for (int q = 0; q < PER_RANK; ++q) {
+                const int rk = q * T + tid;
+                if (rk >= nb) continue;
+                const uint32_t i = my_i[q];
+                const long long o = (long long)b * p.k + blo + rk;
+                p.values[o] = scores[i];
+                p.indices[o] = remap ? remap[i] : (int)i;
                 if (p.gathered) {
                     if (p.reg) {   // predictor.py:55-56 for the selected rows only: decode(anchor, delta * variances)
-                        float4 bx = decode_ref(anchor_of(p, anc, my_i), mul4(ldg_f4(p.reg + (long long)b * SN + my_i), p.var));
+                        float4 bx = decode_ref(anchor_of(p, anc, i), mul4(ldg_f4(p.reg + (long long)b * SN + i), p.var));
                         p.gathered[o] = p.clip_decoded ? clip01(bx) : bx;
                     } else {
-                        p.gathered[o] = ldg_f4(p.boxes + (long long)b * p.box_stride + my_i);
+                        p.gathered[o] = ldg_f4(p.boxes + (long long)b * p.box_stride + i);
                     }
                 }
             }
@@ -496,7 +581,8 @@ __global__ void __launch_bounds__(PR_THREADS, 1) proposal_kernel(PropParams p) {
         }
 
         // ---- 4b. greedy NMS rounds over this batch ---------------------------------------------
-        sidx[tid] = my_i;
+#pragma unroll
+        for (int q = 0; q < PER_RANK; ++q) sidx[q * T + tid] = my_i[q];
         __syncthreads();
         auto fetch = [&](int pos, float4& a, float4& d, uint32_t& idx) {
             if (p.rows_fetched && tid == 0 && pos < nb) atomicAdd(p.rows_fetched, (unsigned long long)min(NMS_CHUNK, nb - pos));
@@ -575,16 +661,19 @@ __global__ void __launch_bounds__(PR_THREADS, 1) proposal_kernel(PropParams p) {
             {   // intra-round predecessor masks over the A survivors: bit j of row i set iff j < i and j suppresses i.
                 // The triangle is folded so that every 16-thread team gets the same number of pairs:
                 // team r takes row iA = r + 1 (iA pairs) and row iB = A - 1 - r (iB pairs) of the compact order.
+                // With T / 16 < 64 teams, team r also takes the folded pair r + T / 16.
                 const int A = sh.nalive;
-                const int r = tid >> 4, sub = tid & 15;
-                const int iA = r + 1, iB = A - 1 - r;
-                const int len = (iA < iB) ? iA + iB : (iA == iB ? iA : 0);
-                for (int e = sub; e < len; e += 16) {
-                    const int i = slot[e < iA ? iA : iB];
-                    const int j = slot[e < iA ? e : e - iA];
-                    if (thr.fast ? nms_suppresses_filtered(cbox[j], carea[j], cbox[i], carea[i], thr)
-                                 : nms_suppresses(cbox[j], carea[j], cbox[i], carea[i], thr))
-                        atomicOr(&mask32[i * 4 + (j >> 5)], 1u << (j & 31));
+                const int sub = tid & 15;
+                for (int r = tid >> 4; r < NMS_CHUNK / 2; r += T / 16) {
+                    const int iA = r + 1, iB = A - 1 - r;
+                    const int len = (iA < iB) ? iA + iB : (iA == iB ? iA : 0);
+                    for (int e = sub; e < len; e += 16) {
+                        const int i = slot[e < iA ? iA : iB];
+                        const int j = slot[e < iA ? e : e - iA];
+                        if (thr.fast ? nms_suppresses_filtered(cbox[j], carea[j], cbox[i], carea[i], thr)
+                                     : nms_suppresses(cbox[j], carea[j], cbox[i], carea[i], thr))
+                            atomicOr(&mask32[i * 4 + (j >> 5)], 1u << (j & 31));
+                    }
                 }
             }
             __syncthreads();
@@ -651,7 +740,7 @@ __global__ void __launch_bounds__(PR_THREADS, 1) proposal_kernel(PropParams p) {
         return;
     }
     // zero padding (TF pads boxes/scores/classes with 0); keep_idx pads with -1
-    for (int rnk = tid; rnk < p.rows; rnk += PR_THREADS) {
+    for (int rnk = tid; rnk < p.rows; rnk += T) {
         const long long o = (long long)b * p.rows + rnk;
         if (rnk >= nkept) {
             p.out_boxes[o] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -1724,7 +1813,8 @@ static size_t cluster_smem_bytes(int cl, int n_staged, int max_out) {
 
 int set_attributes_proposals() {
     const int lim = (int)(227 * 1024 - 4096);
-    TFRPN_CHECK_CUDA(cudaFuncSetAttribute(proposal_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
+    TFRPN_CHECK_CUDA(cudaFuncSetAttribute(proposal_kernel<1024>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
+    TFRPN_CHECK_CUDA(cudaFuncSetAttribute(proposal_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
     TFRPN_CHECK_CUDA(cudaFuncSetAttribute(proposal_cluster_kernel<1, 1024>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
     TFRPN_CHECK_CUDA(cudaFuncSetAttribute(proposal_cluster_kernel<2, 512>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
     TFRPN_CHECK_CUDA(cudaFuncSetAttribute(proposal_cluster_kernel<2, 1024>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
@@ -1742,7 +1832,7 @@ int set_attributes_proposals() {
 // as the batch alone can fill the GPU -- and with the target kernels and other steps running beside it -- the one-CTA
 // kernel gives more images/s AND the lower step latency (bench.py at C2: 1.42 M images/s, p50 67.6 us against 1.34 M,
 // 71.7 us with 2 x 512; C4, B = 32: 196 k against 173 k with 8 x 256).  Hence: B <= 8 -> 8 CTAs x 256 threads per
-// image, larger batches -> one 1024-thread CTA per image.  TFRPN_PROP_CLUSTER = 10 * t + cl forces a shape (A/B
+// image, larger batches -> one CTA per image (proposal_kernel<T>, T picked in launch_one).  TFRPN_PROP_CLUSTER = 10 * t + cl forces a shape (A/B
 // switch): cl = 0 one-CTA kernel, 1 / 2 / 4 / 8 CTAs per image; t selects the threads per CTA.
 static void pick_cluster(tfrpn_handle h, int B, int& cl, int& threads) {
     const int v = h->opts.prop_cluster;
@@ -2183,6 +2273,11 @@ __global__ void __launch_bounds__(256) gather_rows_kernel(const float4* __restri
     if (counter && t == 0) atomicAdd(counter, (unsigned long long)n);
 }
 
+// Every launch of the one-CTA kernel comes through here: the proposal stage, tfrpn_topk / tfrpn_nms (the large-N
+// prefilter's compact launch and its redo of flagged images included) and the per-class launch of
+// tfrpn_nms_multiclass.  Threads per CTA: 512 whenever two such CTAs, each with this launch's dynamic shared memory,
+// fit one SM -- an image then holds half an SM's threads and registers, and the two CTAs fill each other's barrier
+// gaps -- else 1024 (large staged N, large max_out).  TFRPN_PROP_THREADS = 512 | 1024 forces one build (A/B switch).
 static int launch_one(tfrpn_handle h, PropParams& p, int B, cudaStream_t st) {
     p.mo_pad = (p.max_out + 3) & ~3;
     int cl = 0, threads = 1024;
@@ -2193,8 +2288,15 @@ static int launch_one(tfrpn_handle h, PropParams& p, int B, cudaStream_t st) {
     if (smem > PROP_SMEM_LIMIT)
         return fail(TFRPN_ERR_UNSUPPORTED, "NMS: %d output rows need %zu B of shared memory (> %zu)", p.max_out, smem,
                     PROP_SMEM_LIMIT);
+    threads = h->opts.prop_threads;
+    if (threads != 512 && threads != 1024) {
+        int per_sm = 0;
+        TFRPN_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, proposal_kernel<512>, 512, smem));
+        threads = per_sm >= 2 ? 512 : 1024;
+    }
     prof_begin(h, TFRPN_K_PROPOSAL, st);
-    proposal_kernel<<<B, PR_THREADS, smem, st>>>(p);
+    if (threads == 512) proposal_kernel<512><<<B, 512, smem, st>>>(p);
+    else proposal_kernel<1024><<<B, 1024, smem, st>>>(p);
     prof_end(h, st);
     TFRPN_AFTER_LAUNCH("proposal_kernel");
     return 0;
