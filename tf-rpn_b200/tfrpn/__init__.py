@@ -10,5 +10,6 @@ from .utils import bbox_utils, data_utils, train_utils  # noqa: F401
 from .proposals import generate_proposals, predict_top_boxes  # noqa: F401
 from .pipeline import HostPipeline, prefetching_rpn_generator  # noqa: F401
 from .evaluation import DetectionMAP, ProposalRecall, detection_map, proposal_recall  # noqa: F401
+from .roi_targets import RoiTargets, roi_target_cfg, roi_targets  # noqa: F401
 
 __version__ = "0.1.0"

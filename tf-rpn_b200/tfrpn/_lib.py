@@ -58,6 +58,13 @@ class MapState(C.Structure):
                 ("overflow", C.c_void_p)]
 
 
+class RoiTargetCfg(C.Structure):
+    _fields_ = [("num_classes", C.c_int32), ("total_pos", C.c_int32), ("total_neg", C.c_int32),
+                ("fg_iou_threshold", C.c_float), ("bg_iou_high", C.c_float), ("bg_iou_low", C.c_float),
+                ("variances", C.c_float * 4), ("append_gt", C.c_int32), ("image_offset", C.c_int32),
+                ("seed", C.c_uint64), ("offset", C.c_uint64)]
+
+
 class StepBuffers(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("gt_boxes", "gt_labels", "rpn_reg", "rpn_cls", "deltas", "labels",
                                           "out_boxes", "out_scores", "valid", "keep_idx")]
@@ -89,6 +96,7 @@ PROTOTYPES = {
     "tfrpn_rpn_targets": (I, [P, P, P, P, I, I, I, C.POINTER(TargetCfg), P, P, C.POINTER(TargetDebug), P]),
     "tfrpn_rpn_targets_compact": (I, [P, P, P, P, I, I, I, C.POINTER(TargetCfg), P, P, P, P]),
     "tfrpn_expand_targets_host": (I, [P, P, I, I, I, P, I, P]),
+    "tfrpn_roi_targets": (I, [P, P, P, P, P, I, I, I, C.POINTER(RoiTargetCfg), P, P, P, P, P, P, P, P]),
     "tfrpn_select_mask": (I, [P, P, P, I, I, I, C.c_uint64, C.c_uint64, I, I, P, P]),
     "tfrpn_rpn_losses": (I, [P, P, P, P, P, I, I, C.c_float, P, P, P, P]),
     "tfrpn_topk": (I, [P, P, I, I, I, P, P, P, I, P, P]),
