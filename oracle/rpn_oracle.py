@@ -49,6 +49,12 @@ def _pair(v):
     return int(v), int(v)
 
 
+def clip01(x):
+    """The library's clip to [0, 1] (include/tfrpn.h): min(max(x, 0), 1) with NaN-ignoring max / min, so NaN -> 0.
+    np.clip would keep NaN.  TF's GPU minimum / maximum also send NaN to the other operand; its CPU kernels keep it."""
+    return np.fmin(np.fmax(np.asarray(x, F32), F32(0)), F32(1))
+
+
 # --------------------------------------------------------------------------------------
 # anchors (utils/bbox_utils.py:3-46)
 # --------------------------------------------------------------------------------------
@@ -88,7 +94,7 @@ def generate_anchors(hp):
     base = generate_base_anchors(hp)
     anchors = base.reshape(1, -1, 4) + grid_map.reshape(-1, 1, 4)
     anchors = anchors.reshape(-1, 4).astype(F32)
-    return np.clip(anchors, F32(0), F32(1))
+    return clip01(anchors)
 
 
 # --------------------------------------------------------------------------------------
@@ -373,7 +379,7 @@ def combined_non_max_suppression(boxes, scores, max_output_size_per_class, max_t
         nv[b] = len(cand)
         for r, (_, c, _, i) in enumerate(cand):
             kept = boxes[b, i, c if q > 1 else 0, :]
-            nb[b, r] = np.clip(kept, F32(0), F32(1)) if clip_boxes else kept
+            nb[b, r] = clip01(kept) if clip_boxes else kept
             ns[b, r] = scores[b, i, c]
             nc[b, r] = F32(c)
             ni[b, r] = i
@@ -401,7 +407,7 @@ def generate_proposals(rpn_reg, rpn_cls, anchors, hp, pre_nms_topn=None, post_nm
     thr = nms_iou_threshold if nms_iou_threshold is not None else hp.get("nms_iou_threshold", 0.7)
     deltas = deltas * np.asarray(hp["variances"], F32)                # predictor.py:55
     boxes = get_bboxes_from_deltas(anchors, deltas)                   # predictor.py:56
-    boxes = np.clip(boxes, F32(0), F32(1))
+    boxes = clip01(boxes)
     top_scores, top_idx = top_k(scores, k)                            # predictor.py:58
     top_boxes = np.take_along_axis(boxes, top_idx[..., None].astype(np.int64), axis=1)  # :60
     nb, ns, _, nv, ni = combined_non_max_suppression(

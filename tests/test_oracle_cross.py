@@ -89,3 +89,38 @@ def test_select_topk_proposals_numpy_vs_c():
     cb, cs, cv, ck = CO.proposals(reg, cls, anchors, hp)
     ob, os_, ov, ok = O.generate_proposals(reg, cls, anchors, hp)
     assert np.array_equal(cv, ov) and np.array_equal(ck, ok) and np.array_equal(cs, os_) and close(cb, ob)
+
+
+def test_clip_sends_nan_to_zero_numpy_vs_c():
+    """Both restatements clip to [0, 1] with NaN-ignoring max / min (include/tfrpn.h): a NaN coordinate becomes 0.
+    NaN regressions on the best-scoring rows and a zero-extent anchor whose exp overflows (0 * inf = NaN) reach the
+    proposal stage's clip; NaN boxes among the NMS inputs reach its clip_boxes.  A NaN box neither suppresses nor is
+    suppressed on either side, so the keep lists agree too."""
+    from tfrpn import synthetic
+    rng = np.random.default_rng(12)
+    hp = O.get_hyper_params("vgg16")
+    anchors = O.generate_anchors(hp)
+    anchors[7] = [0.4, 0.4, 0.4, 0.4]                       # zero extent
+    reg, cls = synthetic.head_outputs(rng, 2, 31, 31, 9)
+    reg = reg.reshape(2, -1, 4)
+    cls = cls.reshape(2, -1)
+    top = np.argsort(-cls, axis=1)[:, :40]
+    reg[0, top[0, ::3], 1] = np.nan
+    reg[1, top[1, ::2]] = np.nan
+    reg[:, 7, 2:] = 1000.0
+    cls[:, 7] = 1.0
+    with np.errstate(invalid="ignore", over="ignore"):
+        ob, os_, ov, ok = O.generate_proposals(reg, cls, anchors, hp)
+    cb, cs, cv, ck = CO.proposals(reg, cls, anchors, hp)
+    assert not np.isnan(ob).any() and np.array_equal(ok[:, 0], [7, 7])
+    assert np.array_equal(cv, ov) and np.array_equal(ck, ok) and np.array_equal(cs, os_) and close(cb, ob)
+    boxes, scores = synthetic.nms_boxes(rng, 2, 300)
+    boxes[0, ::5, 0] = np.nan
+    boxes[1, ::7] = np.nan
+    boxes[1, 1::7, 3] = np.nan
+    r = CO.nms(boxes, scores, 100, 120, 0.5)
+    with np.errstate(invalid="ignore"):
+        w = O.combined_non_max_suppression(boxes[:, :, None], scores[:, :, None], 100, 120, 0.5, return_indices=True)
+    assert not np.isnan(w[0]).any()
+    assert np.array_equal(r[3], w[3]) and np.array_equal(r[4], w[4])
+    assert np.array_equal(bits(r[0]), bits(w[0])) and np.array_equal(bits(r[1]), bits(w[1]))
