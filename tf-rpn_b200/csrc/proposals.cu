@@ -259,6 +259,149 @@ __device__ __forceinline__ unsigned nms_maybe2(float4 c, f32x2 ca2, float4 k0, f
 __device__ __forceinline__ bool nms_suppresses_filtered(float4 ci, float ai, float4 cj, float aj, const IouThreshold& t) {
     return nms_maybe(ci, ai, cj, aj, t.lo_s) && nms_suppresses_fast(ci, ai, cj, aj, t);
 }
+// the pair test for boxes staged by canonical_box
+__device__ __forceinline__ bool pair_suppresses(const IouThreshold& thr, float4 ci, float ai, float4 cj, float aj) {
+    return thr.fast ? nms_suppresses_filtered(ci, ai, cj, aj, thr) : nms_suppresses(ci, ai, cj, aj, thr);
+}
+
+// canonical box (ymin, xmin, ymax, xmax) and area of a raw box, as the pair tests take them
+__device__ __forceinline__ void canonical_box(float4 raw, const IouThreshold& thr, float4& c, float& ca) {
+    c = make_float4(fminf(raw.x, raw.z), fminf(raw.y, raw.w), fmaxf(raw.x, raw.z), fmaxf(raw.y, raw.w));
+    ca = __fmul_rn(__fsub_rn(c.z, c.x), __fsub_rn(c.w, c.y));
+    if (thr.fast && !(ca > 0.0f)) { c = TFRPN_FAR_BOX; ca = 0.0f; }   // see nms_suppresses_fast
+}
+
+// candidate (cb, ca) against the kept boxes j = first, first + stride, ... < nkept: G (2 or 4) independent tests per
+// iteration (the tests are latency chains; the early exit is checked once per group)
+template <int G>
+__device__ __forceinline__ bool kept_list_suppresses(float4 cb, float ca, const float4* kbox, const float* karea, int first,
+                                                     int stride, int nkept, const IouThreshold& thr) {
+    static_assert(G == 2 || G == 4, "kept_list_suppresses: groups of 2 or 4");
+    bool dead = false;
+    int j = first;
+    if (thr.fast) {
+        const f32x2 ca2 = pack2(ca, ca), lo2 = pack2(thr.lo_s, thr.lo_s);
+        for (; j + (G - 1) * stride < nkept && !dead; j += G * stride) {
+            unsigned m = nms_maybe2(cb, ca2, kbox[j], karea[j], kbox[j + stride], karea[j + stride], lo2);
+            if (G == 4)
+                m |= nms_maybe2(cb, ca2, kbox[j + 2 * stride], karea[j + 2 * stride], kbox[j + 3 * stride], karea[j + 3 * stride],
+                                lo2) << 2;
+            if (m != 0u) {   // rare: the exact test for the pairs that passed
+#pragma unroll
+                for (int u = 0; u < G; ++u)
+                    if (!dead && ((m >> u) & 1u)) dead = nms_suppresses_fast(cb, ca, kbox[j + u * stride], karea[j + u * stride], thr);
+            }
+        }
+        if (G == 2) { if (!dead && j < nkept) dead = nms_suppresses_filtered(cb, ca, kbox[j], karea[j], thr); }
+        else for (; j < nkept && !dead; j += stride) dead = nms_suppresses_filtered(cb, ca, kbox[j], karea[j], thr);
+    } else {
+        for (; j < nkept && !dead; j += stride) dead = nms_suppresses(cb, ca, kbox[j], karea[j], thr);
+    }
+    return dead;
+}
+
+// Resolves a round of NMS_CHUNK candidates in warp 0, in parallel sweeps (same result as the sequential greedy loop):
+// an undecided candidate is REMOVED if a kept predecessor suppresses it, KEPT if no undecided predecessor does, else
+// stays undecided.  Lane l owns candidates l, 32+l, 64+l, 96+l, so ballot word q is exactly bits [32q, 32q+32).
+// m4[c]: the predecessor words of candidate c inside the round; U: the candidates that enter the sweeps (those the kept
+// list suppresses are left out).  Kept candidates take consecutive output slots from nkept in score order, capped at
+// max_out: slot[c] = its slot or -1, kept[0..3] (if not null) = the kept words after the cap.  Returns the number of
+// candidates kept.
+__device__ __forceinline__ int resolve_round(const uint4* m4, unsigned (&U)[4], int nkept, int max_out, int* slot,
+                                             unsigned* kept) {
+    const int lane = lane_id();
+    uint4 pr[4];
+    unsigned Kp[4] = {0u, 0u, 0u, 0u};
+#pragma unroll
+    for (int q = 0; q < 4; ++q) pr[q] = m4[q * 32 + lane];
+    while ((U[0] | U[1] | U[2] | U[3]) != 0u) {
+        unsigned nU[4], nK[4];
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            const bool und = (U[q] >> lane) & 1u;
+            const unsigned hitK = (pr[q].x & Kp[0]) | (pr[q].y & Kp[1]) | (pr[q].z & Kp[2]) | (pr[q].w & Kp[3]);
+            const unsigned hitU = (pr[q].x & U[0]) | (pr[q].y & U[1]) | (pr[q].z & U[2]) | (pr[q].w & U[3]);
+            nK[q] = __ballot_sync(0xffffffffu, und && hitK == 0u && hitU == 0u);
+            nU[q] = __ballot_sync(0xffffffffu, und && hitK == 0u && hitU != 0u);
+        }
+#pragma unroll
+        for (int q = 0; q < 4; ++q) { Kp[q] |= nK[q]; U[q] = nU[q]; }
+    }
+    const int allowed = max_out - nkept;
+    int before = 0;
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+        const int rank = before + __popc(Kp[q] & ((1u << lane) - 1u));
+        const bool k = ((Kp[q] >> lane) & 1u) && rank < allowed;
+        slot[q * 32 + lane] = k ? nkept + rank : -1;
+        if (kept) kept[q] = __ballot_sync(0xffffffffu, k);
+        before += __popc(Kp[q]);
+    }
+    return min(before, allowed);
+}
+
+// warp-aggregated append: the lanes with `pred` store `v` at consecutive positions of dst, reserved with one atomicAdd
+// on *cursor (all lanes call)
+__device__ __forceinline__ void warp_append(bool pred, unsigned long long v, unsigned int* cursor, unsigned long long* dst) {
+    const int lane = lane_id();
+    const unsigned bal = __ballot_sync(0xffffffffu, pred);
+    if (bal != 0u) {
+        unsigned int pos0 = 0;
+        if (lane == __ffs(bal) - 1) pos0 = atomicAdd(cursor, (unsigned)__popc(bal));
+        pos0 = __shfl_sync(0xffffffffu, pos0, __ffs(bal) - 1);
+        if (pred) dst[pos0 + __popc(bal & ((1u << lane) - 1u))] = v;
+    }
+}
+
+// decoded box of an entry (predictor.py:55-56): decode(anchor, delta * variances), clipped to [0, 1] if asked
+__device__ __forceinline__ float4 decoded_box(const PropParams& p, float4 anchor, float4 delta) {
+    const float4 raw = decode_ref(anchor, mul4(delta, p.var));
+    return p.clip_decoded ? clip01(raw) : raw;
+}
+// raw (decoded, optionally clipped) box of the entry `idx` at rank `rank` of image b; ranks below compact_rows read
+// their regression row from reg_compact
+__device__ __forceinline__ float4 ranked_raw_box(const PropParams& p, int b, int rank, uint32_t idx) {
+    if (p.mode == MODE_PROPOSALS) {
+        const float4 row = (p.reg_compact && rank < p.compact_rows)
+                               ? ldg_f4(p.reg_compact + (long long)b * p.compact_stride + rank)
+                               : ldg_f4(p.reg + (long long)b * p.N + idx);
+        const float4* anc = p.anchors + (p.anchors_batched ? (long long)b * p.N : 0LL);
+        return decoded_box(p, anchor_of(p, anc, idx), row);
+    }
+    return ldg_f4(p.boxes + (long long)b * p.box_stride + idx);
+}
+
+// MODE_TOPK output row o of image b: score and index of entry i, and its gathered or decoded box if asked
+__device__ __forceinline__ void write_topk_row(const PropParams& p, int b, long long o, uint32_t i, const float* scores,
+                                               const float4* anc, const int* remap) {
+    p.values[o] = scores[i];
+    p.indices[o] = remap ? remap[i] : (int)i;
+    if (p.gathered) {
+        if (p.reg) p.gathered[o] = decoded_box(p, anchor_of(p, anc, i), ldg_f4(p.reg + (long long)b * p.N + i));
+        else p.gathered[o] = ldg_f4(p.boxes + (long long)b * p.box_stride + i);
+    }
+}
+// output slot s of image b for the kept entry idx with raw box `raw`
+__device__ __forceinline__ void write_kept_row(const PropParams& p, int b, int s, float4 raw, const float* scores, uint32_t idx,
+                                               const int* remap) {
+    const long long o = (long long)b * p.rows + s;
+    p.out_boxes[o] = p.clip_out ? clip01(raw) : raw;
+    p.out_scores[o] = scores[idx];
+    if (p.keep_idx) p.keep_idx[o] = remap ? remap[idx] : (int)idx;
+}
+// output rows first, first + stride, ... of image b: zero padding past nkept (TF pads boxes/scores/classes with 0;
+// keep_idx pads with -1), and the class column
+__device__ __forceinline__ void pad_outputs(const PropParams& p, int b, int nkept, int first, int stride) {
+    for (int rnk = first; rnk < p.rows; rnk += stride) {
+        const long long o = (long long)b * p.rows + rnk;
+        if (rnk >= nkept) {
+            p.out_boxes[o] = make_float4(0.f, 0.f, 0.f, 0.f);
+            p.out_scores[o] = 0.0f;
+            if (p.keep_idx) p.keep_idx[o] = -1;
+        }
+        if (p.out_classes) p.out_classes[o] = 0.0f;
+    }
+}
 
 // descending bitonic sort of BATCH composites, one per thread of a BATCH-thread CTA; thread t ends with rank t.
 // Strides < 32 use shuffles; strides >= 32 go through a double-buffered shared array (1 barrier each).
@@ -420,15 +563,7 @@ __global__ void __launch_bounds__(T, BATCH / T) proposal_kernel(PropParams p) {
                         in = eligible(c) && c >= prefix;
                     }
                     if (in && ((c ^ prefix) & himask) == 0ull) atomicAdd(&hist[(unsigned)(c >> shift) & dmask], 1u);
-                    if (listing) {
-                        const unsigned bal = __ballot_sync(0xffffffffu, in);
-                        if (bal != 0u) {
-                            unsigned int pos0 = 0;
-                            if (lane == __ffs(bal) - 1) pos0 = atomicAdd(&sh.lcount, (unsigned)__popc(bal));
-                            pos0 = __shfl_sync(0xffffffffu, pos0, __ffs(bal) - 1);
-                            if (in) sortbuf[pos0 + __popc(bal & ((1u << lane) - 1u))] = c;
-                        }
-                    }
+                    if (listing) warp_append(in, c, &sh.lcount, sortbuf);
                 }
             }
             __syncthreads();                            // histogram (and list) complete
@@ -473,13 +608,7 @@ __global__ void __launch_bounds__(T, BATCH / T) proposal_kernel(PropParams p) {
                     c = make_comp(key_at(i), i);
                     take = eligible(c) && c >= tau;
                 }
-                const unsigned bal = __ballot_sync(0xffffffffu, take);
-                if (bal != 0u) {
-                    unsigned int pos0 = 0;
-                    if (lane == __ffs(bal) - 1) pos0 = atomicAdd(&sh.lcount, (unsigned)__popc(bal));
-                    pos0 = __shfl_sync(0xffffffffu, pos0, __ffs(bal) - 1);
-                    if (take) sortbuf[pos0 + __popc(bal & ((1u << lane) - 1u))] = c;
-                }
+                warp_append(take, c, &sh.lcount, sortbuf);
             }
             __syncthreads();
             nl = (int)sh.lcount;
@@ -562,19 +691,7 @@ __global__ void __launch_bounds__(T, BATCH / T) proposal_kernel(PropParams p) {
 #pragma unroll
             for (int q = 0; q < PER_RANK; ++q) {
                 const int rk = q * T + tid;
-                if (rk >= nb) continue;
-                const uint32_t i = my_i[q];
-                const long long o = (long long)b * p.k + blo + rk;
-                p.values[o] = scores[i];
-                p.indices[o] = remap ? remap[i] : (int)i;
-                if (p.gathered) {
-                    if (p.reg) {   // predictor.py:55-56 for the selected rows only: decode(anchor, delta * variances)
-                        float4 bx = decode_ref(anchor_of(p, anc, i), mul4(ldg_f4(p.reg + (long long)b * SN + i), p.var));
-                        p.gathered[o] = p.clip_decoded ? clip01(bx) : bx;
-                    } else {
-                        p.gathered[o] = ldg_f4(p.boxes + (long long)b * p.box_stride + i);
-                    }
-                }
+                if (rk < nb) write_topk_row(p, b, (long long)b * p.k + blo + rk, my_i[q], scores, anc, remap);
             }
             __syncthreads();   // sortbuf is rewritten by the next batch
             continue;
@@ -604,13 +721,10 @@ __global__ void __launch_bounds__(T, BATCH / T) proposal_kernel(PropParams p) {
             float4 raw = na;
             const uint32_t my_idx = nidx;
             if (tid < C) {
-                if (p.mode == MODE_PROPOSALS) {
-                    raw = decode_ref(na, mul4(nd, p.var));                               // predictor.py:55-56
-                    if (p.clip_decoded) raw = clip01(raw);
-                }
-                float4 c = make_float4(fminf(raw.x, raw.z), fminf(raw.y, raw.w), fmaxf(raw.x, raw.z), fmaxf(raw.y, raw.w));
-                float ca = __fmul_rn(__fsub_rn(c.z, c.x), __fsub_rn(c.w, c.y));
-                if (thr.fast && !(ca > 0.0f)) { c = TFRPN_FAR_BOX; ca = 0.0f; }   // see nms_suppresses_fast
+                if (p.mode == MODE_PROPOSALS) raw = decoded_box(p, na, nd);
+                float4 c;
+                float ca;
+                canonical_box(raw, thr, c, ca);
                 cbox[tid] = c;
                 carea[tid] = ca;
                 alive[tid] = 1u;
@@ -621,26 +735,7 @@ __global__ void __launch_bounds__(T, BATCH / T) proposal_kernel(PropParams p) {
             fetch(pos + NMS_CHUNK, na, nd, nidx);   // in flight during the tests below
             {   // candidates vs kept list: thread = (candidate c, part), kept j strided by NMS_PARTS
                 const int c = tid & (NMS_CHUNK - 1), part = tid >> 7;
-                if (c < C) {
-                    const float4 cb = cbox[c];
-                    const float ca = carea[c];
-                    bool dead = false;
-                    if (thr.fast) {
-                        int j = part;
-                        const f32x2 ca2 = pack2(ca, ca), lo2 = pack2(thr.lo_s, thr.lo_s);
-                        for (; j + NMS_PARTS < nkept && !dead; j += 2 * NMS_PARTS) {
-                            const unsigned m = nms_maybe2(cb, ca2, kbox[j], karea[j], kbox[j + NMS_PARTS], karea[j + NMS_PARTS], lo2);
-                            if (m != 0u) {   // rare: the exact test for the pairs that passed
-                                if (m & 1u) dead = nms_suppresses_fast(cb, ca, kbox[j], karea[j], thr);
-                                if (!dead && (m & 2u)) dead = nms_suppresses_fast(cb, ca, kbox[j + NMS_PARTS], karea[j + NMS_PARTS], thr);
-                            }
-                        }
-                        if (!dead && j < nkept) dead = nms_suppresses_filtered(cb, ca, kbox[j], karea[j], thr);
-                    } else {
-                        for (int j = part; j < nkept && !dead; j += NMS_PARTS) dead = nms_suppresses(cb, ca, kbox[j], karea[j], thr);
-                    }
-                    if (dead) alive[c] = 0u;
-                }
+                if (c < C && kept_list_suppresses<2>(cbox[c], carea[c], kbox, karea, part, NMS_PARTS, nkept, thr)) alive[c] = 0u;
             }
             __syncthreads();
             PH(7);
@@ -670,52 +765,21 @@ __global__ void __launch_bounds__(T, BATCH / T) proposal_kernel(PropParams p) {
                     for (int e = sub; e < len; e += 16) {
                         const int i = slot[e < iA ? iA : iB];
                         const int j = slot[e < iA ? e : e - iA];
-                        if (thr.fast ? nms_suppresses_filtered(cbox[j], carea[j], cbox[i], carea[i], thr)
-                                     : nms_suppresses(cbox[j], carea[j], cbox[i], carea[i], thr))
-                            atomicOr(&mask32[i * 4 + (j >> 5)], 1u << (j & 31));
+                        if (pair_suppresses(thr, cbox[j], carea[j], cbox[i], carea[i])) atomicOr(&mask32[i * 4 + (j >> 5)], 1u << (j & 31));
                     }
                 }
             }
             __syncthreads();
             PH(9);
-            if (warp == 0) {
-                // Resolve the round in parallel sweeps (same result as the sequential greedy loop):
-                // an undecided candidate is REMOVED if a kept predecessor suppresses it, KEPT if no
-                // undecided predecessor suppresses it, else stays undecided.  Lane l owns candidates
-                // l, 32+l, 64+l, 96+l, so ballot word q is exactly bits [32q, 32q+32).
-                const uint4* m4 = reinterpret_cast<const uint4*>(mask32);
-                uint4 pr[4];
-                unsigned U[4], Kp[4] = {0u, 0u, 0u, 0u};
+            if (warp == 0) {   // the round's greedy order, over the candidates that survived the kept list
+                unsigned U[4];
 #pragma unroll
                 for (int q = 0; q < 4; ++q) {
                     const int c = q * 32 + lane;
-                    pr[q] = m4[c];
                     U[q] = __ballot_sync(0xffffffffu, c < C && alive[c] != 0u);
                 }
-                while ((U[0] | U[1] | U[2] | U[3]) != 0u) {
-                    unsigned nU[4], nK[4];
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        const bool und = (U[q] >> lane) & 1u;
-                        const unsigned hitK = (pr[q].x & Kp[0]) | (pr[q].y & Kp[1]) | (pr[q].z & Kp[2]) | (pr[q].w & Kp[3]);
-                        const unsigned hitU = (pr[q].x & U[0]) | (pr[q].y & U[1]) | (pr[q].z & U[2]) | (pr[q].w & U[3]);
-                        nK[q] = __ballot_sync(0xffffffffu, und && hitK == 0u && hitU == 0u);
-                        nU[q] = __ballot_sync(0xffffffffu, und && hitK == 0u && hitU != 0u);
-                    }
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) { Kp[q] |= nK[q]; U[q] = nU[q]; }
-                }
-                // kept candidates take consecutive output slots in score order, capped at max_out
-                const int allowed = p.max_out - nkept;
-                int before = 0;
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    const int rank = before + __popc(Kp[q] & ((1u << lane) - 1u));
-                    const bool kept = ((Kp[q] >> lane) & 1u) && rank < allowed;
-                    slot[q * 32 + lane] = kept ? nkept + rank : -1;
-                    before += __popc(Kp[q]);
-                }
-                if (lane == 0) sh.nk = min(before, allowed);
+                const int nk = resolve_round(reinterpret_cast<const uint4*>(mask32), U, nkept, p.max_out, slot, nullptr);
+                if (lane == 0) sh.nk = nk;
             }
             __syncthreads();
             PH(10);
@@ -723,10 +787,7 @@ __global__ void __launch_bounds__(T, BATCH / T) proposal_kernel(PropParams p) {
                 const int s = slot[tid];
                 kbox[s] = cbox[tid];
                 karea[s] = carea[tid];
-                const long long o = (long long)b * p.rows + s;
-                p.out_boxes[o] = p.clip_out ? clip01(raw) : raw;
-                p.out_scores[o] = scores[my_idx];
-                if (p.keep_idx) p.keep_idx[o] = remap ? remap[my_idx] : (int)my_idx;
+                write_kept_row(p, b, s, raw, scores, my_idx, remap);
             }
             nkept += sh.nk;
             __syncthreads();
@@ -739,16 +800,7 @@ __global__ void __launch_bounds__(T, BATCH / T) proposal_kernel(PropParams p) {
         if (tid == 0) p.flags_out[b] = 1;
         return;
     }
-    // zero padding (TF pads boxes/scores/classes with 0); keep_idx pads with -1
-    for (int rnk = tid; rnk < p.rows; rnk += T) {
-        const long long o = (long long)b * p.rows + rnk;
-        if (rnk >= nkept) {
-            p.out_boxes[o] = make_float4(0.f, 0.f, 0.f, 0.f);
-            p.out_scores[o] = 0.0f;
-            if (p.keep_idx) p.keep_idx[o] = -1;
-        }
-        if (p.out_classes) p.out_classes[o] = 0.0f;
-    }
+    pad_outputs(p, b, nkept, tid, T);
     if (tid == 0) p.valid[b] = nkept;
     PH(12);
     PH_FLUSH;
@@ -831,31 +883,6 @@ __device__ __forceinline__ unsigned long long bitonic_sort_desc_s(unsigned long 
         }
     }
     return v;
-}
-
-// candidate (cb, ca) against the kept boxes j = first, first + stride, ... < nkept: four independent tests per
-// iteration (the tests are latency chains; the early exit is checked once per group)
-__device__ __forceinline__ bool kept_list_suppresses(float4 cb, float ca, const float4* kbox, const float* karea, int first,
-                                                     int stride, int nkept, const IouThreshold& thr) {
-    bool dead = false;
-    int j = first;
-    if (thr.fast) {
-        const f32x2 ca2 = pack2(ca, ca), lo2 = pack2(thr.lo_s, thr.lo_s);
-        for (; j + 3 * stride < nkept && !dead; j += 4 * stride) {
-            const unsigned m = nms_maybe2(cb, ca2, kbox[j], karea[j], kbox[j + stride], karea[j + stride], lo2) |
-                               (nms_maybe2(cb, ca2, kbox[j + 2 * stride], karea[j + 2 * stride], kbox[j + 3 * stride],
-                                           karea[j + 3 * stride], lo2) << 2);
-            if (m != 0u) {   // rare: the exact test for the pairs that passed
-#pragma unroll
-                for (int u = 0; u < 4; ++u)
-                    if (!dead && ((m >> u) & 1u)) dead = nms_suppresses_fast(cb, ca, kbox[j + u * stride], karea[j + u * stride], thr);
-            }
-        }
-        for (; j < nkept && !dead; j += stride) dead = nms_suppresses_filtered(cb, ca, kbox[j], karea[j], thr);
-    } else {
-        for (; j < nkept && !dead; j += stride) dead = nms_suppresses(cb, ca, kbox[j], karea[j], thr);
-    }
-    return dead;
 }
 
 // CL CTAs x T threads per image; S = 1024 / CL sort slots per CTA (T >= S, T >= 128)
@@ -1138,19 +1165,7 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(T, (T <= 512 && CL 
 
         // ---- 4a. top-k outputs (predictor.py:58-60) -------------------------------------------------
         if (p.mode == MODE_TOPK) {
-            if (real) {
-                const long long o = (long long)b * p.k + lo + rank;
-                p.values[o] = scores[my_i];
-                p.indices[o] = remap ? remap[my_i] : (int)my_i;
-                if (p.gathered) {
-                    if (p.reg) {
-                        float4 bx = decode_ref(anchor_of(p, anc, my_i), mul4(ldg_f4(p.reg + (long long)b * SN + my_i), p.var));
-                        p.gathered[o] = p.clip_decoded ? clip01(bx) : bx;
-                    } else {
-                        p.gathered[o] = ldg_f4(p.boxes + (long long)b * p.box_stride + my_i);
-                    }
-                }
-            }
+            if (real) write_topk_row(p, b, (long long)b * p.k + lo + rank, my_i, scores, anc, remap);
             lo += nb_all; lo_tau = tau; have_lo = true;
             cl_sync<CL>();   // my list / tau are rewritten by the next batch while peers may still be copying them
             continue;
@@ -1161,18 +1176,12 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(T, (T <= 512 && CL 
         if (p.rows_fetched && tid == 0 && crank == 0)
             atomicAdd(p.rows_fetched, (unsigned long long)((p.presorted && p.reg_compact) ? max(nb - p.compact_rows, 0) : nb));
         if (real) {
-            if (p.mode == MODE_PROPOSALS) {
-                const float4 row = (p.presorted && p.reg_compact && rank < p.compact_rows)
-                                       ? ldg_f4(p.reg_compact + (long long)b * p.compact_stride + rank)
-                                       : ldg_f4(p.reg + (long long)b * SN + my_i);
-                raw = decode_ref(anchor_of(p, anc, my_i), mul4(row, p.var));   // predictor.py:55-56
-                if (p.clip_decoded) raw = clip01(raw);
-            } else {
-                raw = ldg_f4(p.boxes + (long long)b * p.box_stride + my_i);
-            }
-            float4 c = make_float4(fminf(raw.x, raw.z), fminf(raw.y, raw.w), fmaxf(raw.x, raw.z), fmaxf(raw.y, raw.w));
-            float ca = __fmul_rn(__fsub_rn(c.z, c.x), __fsub_rn(c.w, c.y));
-            if (thr.fast && !(ca > 0.0f)) { c = TFRPN_FAR_BOX; ca = 0.0f; }   // see nms_suppresses_fast
+            // reg_compact is only set for a presorted launch (proposals_presorted_enqueue), so ranked_raw_box reads it
+            // in presorted launches only
+            raw = ranked_raw_box(p, b, rank, my_i);
+            float4 c;
+            float ca;
+            canonical_box(raw, thr, c, ca);
 #pragma unroll
             for (int q = 0; q < CL; ++q) {
                 cl_peer<CL>(cbox_all, (crank + q) % CL)[rank] = c;
@@ -1191,7 +1200,7 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(T, (T <= 512 && CL 
             const int gt = (int)crank * T + tid;
             if (nkept > 0) {   // candidates vs kept list: thread = (candidate c, part), kept j strided by PARTS
                 const int c = gt & (NMS_CHUNK - 1), part = gt >> 7;
-                if (c < C && kept_list_suppresses(cbox_all[pos + c], carea_all[pos + c], kbox, karea, part, PARTS, nkept, thr))
+                if (c < C && kept_list_suppresses<4>(cbox_all[pos + c], carea_all[pos + c], kbox, karea, part, PARTS, nkept, thr))
                     atomicOr(&sh.dead_w[c >> 5], 1u << (c & 31));
             }
             {   // predecessor masks of the round: bit j of row i set iff j < i and j suppresses i.  Folded triangle
@@ -1203,8 +1212,7 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(T, (T <= 512 && CL 
                 auto pair = [&](int e, int& i, int& j) -> bool {
                     i = e < iA ? iA : iB;
                     j = e < iA ? e : e - iA;
-                    return thr.fast ? nms_suppresses_filtered(cbox_all[pos + j], carea_all[pos + j], cbox_all[pos + i], carea_all[pos + i], thr)
-                                    : nms_suppresses(cbox_all[pos + j], carea_all[pos + j], cbox_all[pos + i], carea_all[pos + i], thr);
+                    return pair_suppresses(thr, cbox_all[pos + j], carea_all[pos + j], cbox_all[pos + i], carea_all[pos + i]);
                 };
                 int e = sub;
                 for (; e + TS < len; e += 2 * TS) {      // two independent tests in flight
@@ -1241,17 +1249,10 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(T, (T <= 512 && CL 
             }
             cl_sync<CL>();                      // the round's barrier
             PH(9);
-            if (warp == 0) {
-                // Resolve the round in parallel sweeps (same result as the sequential greedy loop): an undecided
-                // candidate is REMOVED if a kept predecessor suppresses it, KEPT if no undecided predecessor does,
-                // else stays undecided.  Lane l owns candidates l, 32+l, 64+l, 96+l, so ballot word q is exactly
-                // bits [32q, 32q+32).  Candidates suppressed by the kept list are in neither set.
-                const uint4* m4 = reinterpret_cast<const uint4*>(mk);
-                uint4 pr[4];
-                unsigned U[4], Kp[4] = {0u, 0u, 0u, 0u};
+            if (warp == 0) {   // the round's greedy order; candidates suppressed by the kept list do not enter it
+                unsigned U[4];
 #pragma unroll
                 for (int q = 0; q < 4; ++q) {
-                    pr[q] = m4[q * 32 + lane];
                     unsigned dead_w = 0u;
                     if (nkept > 0) {
 #pragma unroll
@@ -1259,30 +1260,8 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(T, (T <= 512 && CL 
                     }
                     U[q] = __ballot_sync(0xffffffffu, q * 32 + lane < C) & ~dead_w;
                 }
-                while ((U[0] | U[1] | U[2] | U[3]) != 0u) {
-                    unsigned nU[4], nK[4];
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        const bool und = (U[q] >> lane) & 1u;
-                        const unsigned hitK = (pr[q].x & Kp[0]) | (pr[q].y & Kp[1]) | (pr[q].z & Kp[2]) | (pr[q].w & Kp[3]);
-                        const unsigned hitU = (pr[q].x & U[0]) | (pr[q].y & U[1]) | (pr[q].z & U[2]) | (pr[q].w & U[3]);
-                        nK[q] = __ballot_sync(0xffffffffu, und && hitK == 0u && hitU == 0u);
-                        nU[q] = __ballot_sync(0xffffffffu, und && hitK == 0u && hitU != 0u);
-                    }
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) { Kp[q] |= nK[q]; U[q] = nU[q]; }
-                }
-                // kept candidates take consecutive output slots in score order, capped at max_out
-                const int allowed = p.max_out - nkept;
-                int before = 0;
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    const int rk = before + __popc(Kp[q] & ((1u << lane) - 1u));
-                    const bool kept = ((Kp[q] >> lane) & 1u) && rk < allowed;
-                    slot[q * 32 + lane] = kept ? nkept + rk : -1;
-                    before += __popc(Kp[q]);
-                }
-                if (lane == 0) sh.nk = min(before, allowed);
+                const int nk = resolve_round(reinterpret_cast<const uint4*>(mk), U, nkept, p.max_out, slot, nullptr);
+                if (lane == 0) sh.nk = nk;
                 if (lane < 4) sh.dead_w[lane] = 0u;
             }
             __syncthreads();
@@ -1294,12 +1273,7 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(T, (T <= 512 && CL 
             }
             if (real && rank >= pos && rank < pos + C) {   // the owner of a kept candidate writes its outputs
                 const int s = slot[rank - pos];
-                if (s >= 0) {
-                    const long long o = (long long)b * p.rows + s;
-                    p.out_boxes[o] = p.clip_out ? clip01(raw) : raw;
-                    p.out_scores[o] = scores[my_i];
-                    if (p.keep_idx) p.keep_idx[o] = remap ? remap[my_i] : (int)my_i;
-                }
+                if (s >= 0) write_kept_row(p, b, s, raw, scores, my_i, remap);
             }
             nkept += sh.nk;
             __syncthreads();
@@ -1319,16 +1293,7 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(T, (T <= 512 && CL 
         if (tid == 0 && crank == 0) p.flags_out[b] = 1;
         return;
     }
-    // zero padding (TF pads boxes/scores/classes with 0); keep_idx pads with -1
-    for (int rnk = (int)crank * T + tid; rnk < p.rows; rnk += NT) {
-        const long long o = (long long)b * p.rows + rnk;
-        if (rnk >= nkept) {
-            p.out_boxes[o] = make_float4(0.f, 0.f, 0.f, 0.f);
-            p.out_scores[o] = 0.0f;
-            if (p.keep_idx) p.keep_idx[o] = -1;
-        }
-        if (p.out_classes) p.out_classes[o] = 0.0f;
-    }
+    pad_outputs(p, b, nkept, (int)crank * T + tid, NT);
     if (tid == 0 && crank == 0) p.valid[b] = nkept;
     PH(12);
     PH_FLUSH;
@@ -1354,23 +1319,6 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(T, (T <= 512 && CL 
 constexpr int MASK_THREADS = 256;
 constexpr int SWEEP_THREADS = NMS_CHUNK;   // 128
 
-// raw (decoded, optionally clipped) box of the entry `idx` at rank `rank` of image b
-__device__ __forceinline__ float4 ranked_raw_box(const PropParams& p, int b, int rank, uint32_t idx) {
-    if (p.mode == MODE_PROPOSALS) {
-        const float4 row = (p.reg_compact && rank < p.compact_rows)
-                               ? ldg_f4(p.reg_compact + (long long)b * p.compact_stride + rank)
-                               : ldg_f4(p.reg + (long long)b * p.N + idx);
-        const float4* anc = p.anchors + (p.anchors_batched ? (long long)b * p.N : 0LL);
-        float4 raw = decode_ref(anchor_of(p, anc, idx), mul4(row, p.var));   // predictor.py:55-56
-        return p.clip_decoded ? clip01(raw) : raw;
-    }
-    return ldg_f4(p.boxes + (long long)b * p.box_stride + idx);
-}
-__device__ __forceinline__ void canonical_box(float4 raw, const IouThreshold& thr, float4& c, float& ca) {
-    c = make_float4(fminf(raw.x, raw.z), fminf(raw.y, raw.w), fmaxf(raw.x, raw.z), fmaxf(raw.y, raw.w));
-    ca = __fmul_rn(__fsub_rn(c.z, c.x), __fsub_rn(c.w, c.y));
-    if (thr.fast && !(ca > 0.0f)) { c = TFRPN_FAR_BOX; ca = 0.0f; }   // see nms_suppresses_fast
-}
 // ranks of image b the matrix covers, and whether the image has ranks beyond them
 __device__ __forceinline__ int matrix_rows(const PropParams& p, int b, bool& more) {
     int n = p.rank_n[b];
@@ -1469,56 +1417,22 @@ __global__ void __launch_bounds__(SWEEP_THREADS) nms_sweep_kernel(const __grid_c
             if (dead) atomicOr(&dead_s[tid >> 5], 1u << (tid & 31));
         }
         __syncthreads();
-        if (warp == 0) {
-            // the chunk's greedy order resolved in parallel sweeps (see proposal_kernel): lane l owns candidates
-            // l, 32 + l, 64 + l, 96 + l
-            uint4 q4[4];
-            unsigned U[4], Kp[4] = {0u, 0u, 0u, 0u};
+        if (warp == 0) {   // the chunk's greedy order; candidates dead by the earlier chunks do not enter it
+            unsigned U[4], kept[4];
 #pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                q4[q] = pr_s[q * 32 + lane];
-                U[q] = __ballot_sync(0xffffffffu, q * 32 + lane < C) & ~dead_s[q];
-            }
-            while ((U[0] | U[1] | U[2] | U[3]) != 0u) {
-                unsigned nU[4], nK[4];
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    const bool und = (U[q] >> lane) & 1u;
-                    const unsigned hitK = (q4[q].x & Kp[0]) | (q4[q].y & Kp[1]) | (q4[q].z & Kp[2]) | (q4[q].w & Kp[3]);
-                    const unsigned hitU = (q4[q].x & U[0]) | (q4[q].y & U[1]) | (q4[q].z & U[2]) | (q4[q].w & U[3]);
-                    nK[q] = __ballot_sync(0xffffffffu, und && hitK == 0u && hitU == 0u);
-                    nU[q] = __ballot_sync(0xffffffffu, und && hitK == 0u && hitU != 0u);
-                }
-#pragma unroll
-                for (int q = 0; q < 4; ++q) { Kp[q] |= nK[q]; U[q] = nU[q]; }
-            }
-            // kept candidates take consecutive output slots in score order, capped at max_out
-            const int allowed = p.max_out - nkept;
-            int before = 0;
-            unsigned keptw[4];
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                const int rk = before + __popc(Kp[q] & ((1u << lane) - 1u));
-                const bool kept = ((Kp[q] >> lane) & 1u) && rk < allowed;
-                slot[q * 32 + lane] = kept ? nkept + rk : -1;
-                keptw[q] = __ballot_sync(0xffffffffu, kept);
-                before += __popc(Kp[q]);
-            }
+            for (int q = 0; q < 4; ++q) U[q] = __ballot_sync(0xffffffffu, q * 32 + lane < C) & ~dead_s[q];
+            const int nk = resolve_round(pr_s, U, nkept, p.max_out, slot, kept);
             __syncwarp();   // every lane has read dead_s[] above
             if (lane < 4) {
-                kw[w0 + lane] = lane == 0 ? keptw[0] : lane == 1 ? keptw[1] : lane == 2 ? keptw[2] : keptw[3];
+                kw[w0 + lane] = lane == 0 ? kept[0] : lane == 1 ? kept[1] : lane == 2 ? kept[2] : kept[3];
                 dead_s[lane] = 0u;
             }
-            if (lane == 0) s_nk = min(before, allowed);
+            if (lane == 0) s_nk = nk;
         }
         __syncthreads();
-        if (tid < C && slot[tid] >= 0) {
+        if (tid < C && slot[tid] >= 0) {         // (matrix_applies excludes remapped launches)
             const uint32_t idx = (uint32_t)ridx[i];
-            const float4 raw = ranked_raw_box(p, b, i, idx);
-            const long long o = (long long)b * p.rows + slot[tid];
-            p.out_boxes[o] = p.clip_out ? clip01(raw) : raw;
-            p.out_scores[o] = scores[idx];
-            if (p.keep_idx) p.keep_idx[o] = (int)idx;
+            write_kept_row(p, b, slot[tid], ranked_raw_box(p, b, i, idx), scores, idx, nullptr);
         }
         nkept += s_nk;
         __syncthreads();
@@ -1526,15 +1440,7 @@ __global__ void __launch_bounds__(SWEEP_THREADS) nms_sweep_kernel(const __grid_c
     const bool redo = nkept < p.max_out && more;
     if (tid == 0) p.redo_flags[b] = redo ? 1 : 0;
     if (redo) return;                            // the lazy kernel redoes this image and writes all of its outputs
-    for (int rnk = tid; rnk < p.rows; rnk += SWEEP_THREADS) {   // zero padding (TF); keep_idx pads with -1
-        const long long o = (long long)b * p.rows + rnk;
-        if (rnk >= nkept) {
-            p.out_boxes[o] = make_float4(0.f, 0.f, 0.f, 0.f);
-            p.out_scores[o] = 0.0f;
-            if (p.keep_idx) p.keep_idx[o] = -1;
-        }
-        if (p.out_classes) p.out_classes[o] = 0.0f;
-    }
+    pad_outputs(p, b, nkept, tid, SWEEP_THREADS);
     if (tid == 0) p.valid[b] = nkept;
 }
 
@@ -1873,6 +1779,13 @@ static size_t prop_smem_bytes(int n_staged, int max_out) {
     return s + 16;
 }
 constexpr size_t PROP_SMEM_LIMIT = 227 * 1024 - 4096;   // leaves room for the static PropShared
+// the kept list lives in shared memory, which bounds max_out
+static int check_prop_smem(size_t smem, int max_out) {
+    if (smem > PROP_SMEM_LIMIT)
+        return fail(TFRPN_ERR_UNSUPPORTED, "NMS: %d output rows need %zu B of shared memory (> %zu)", max_out, smem,
+                    PROP_SMEM_LIMIT);
+    return 0;
+}
 
 // ------------------------------------------------------------------------------------------------
 // Large-N prefilter.  One CTA per image cannot stream hundreds of thousands of scores several times,
@@ -2229,25 +2142,21 @@ static int launch(tfrpn_handle h, PropParams& p, int B, cudaStream_t st) {
 
 static int launch_cluster(tfrpn_handle h, PropParams& p, int B, int cl, int threads, cudaStream_t st) {
     p.mo_pad = (p.max_out + 3) & ~3;
-    {
-        // (a presorted launch never looks at the scores' order: no staged keys)
-        p.staged = (!p.presorted && cluster_smem_bytes(cl, p.N, p.max_out) <= PROP_SMEM_LIMIT) ? 1 : 0;
-        const size_t smem = cluster_smem_bytes(cl, p.staged ? p.N : 0, p.max_out);
-        if (smem > PROP_SMEM_LIMIT)
-            return fail(TFRPN_ERR_UNSUPPORTED, "NMS: %d output rows need %zu B of shared memory (> %zu)", p.max_out, smem,
-                        PROP_SMEM_LIMIT);
-        prof_begin(h, TFRPN_K_PROPOSAL_CLUSTER, st);
-        if (cl == 8 && threads == 512) proposal_cluster_kernel<8, 512><<<B * 8, 512, smem, st>>>(p);
-        else if (cl == 8) proposal_cluster_kernel<8, 256><<<B * 8, 256, smem, st>>>(p);
-        else if (cl == 4 && threads == 256) proposal_cluster_kernel<4, 256><<<B * 4, 256, smem, st>>>(p);
-        else if (cl == 4) proposal_cluster_kernel<4, 512><<<B * 4, 512, smem, st>>>(p);
-        else if (cl == 2 && threads == 512) proposal_cluster_kernel<2, 512><<<B * 2, 512, smem, st>>>(p);
-        else if (cl == 2) proposal_cluster_kernel<2, 1024><<<B * 2, 1024, smem, st>>>(p);
-        else proposal_cluster_kernel<1, 1024><<<B, 1024, smem, st>>>(p);
-        prof_end(h, st);
-        TFRPN_AFTER_LAUNCH("proposal_cluster_kernel");
-        return 0;
-    }
+    // (a presorted launch never looks at the scores' order: no staged keys)
+    p.staged = (!p.presorted && cluster_smem_bytes(cl, p.N, p.max_out) <= PROP_SMEM_LIMIT) ? 1 : 0;
+    const size_t smem = cluster_smem_bytes(cl, p.staged ? p.N : 0, p.max_out);
+    if (int rc = check_prop_smem(smem, p.max_out)) return rc;
+    prof_begin(h, TFRPN_K_PROPOSAL_CLUSTER, st);
+    if (cl == 8 && threads == 512) proposal_cluster_kernel<8, 512><<<B * 8, 512, smem, st>>>(p);
+    else if (cl == 8) proposal_cluster_kernel<8, 256><<<B * 8, 256, smem, st>>>(p);
+    else if (cl == 4 && threads == 256) proposal_cluster_kernel<4, 256><<<B * 4, 256, smem, st>>>(p);
+    else if (cl == 4) proposal_cluster_kernel<4, 512><<<B * 4, 512, smem, st>>>(p);
+    else if (cl == 2 && threads == 512) proposal_cluster_kernel<2, 512><<<B * 2, 512, smem, st>>>(p);
+    else if (cl == 2) proposal_cluster_kernel<2, 1024><<<B * 2, 1024, smem, st>>>(p);
+    else proposal_cluster_kernel<1, 1024><<<B, 1024, smem, st>>>(p);
+    prof_end(h, st);
+    TFRPN_AFTER_LAUNCH("proposal_cluster_kernel");
+    return 0;
 }
 
 // Device-side variant of the two-phase gather (pipeline.cu): the candidate rows of a PAGE-LOCKED host tensor, in rank
@@ -2285,9 +2194,7 @@ static int launch_one(tfrpn_handle h, PropParams& p, int B, cudaStream_t st) {
     if (cl) return launch_cluster(h, p, B, cl, threads, st);
     p.staged = prop_smem_bytes(p.N, p.max_out) <= PROP_SMEM_LIMIT ? 1 : 0;
     const size_t smem = prop_smem_bytes(p.staged ? p.N : 0, p.max_out);
-    if (smem > PROP_SMEM_LIMIT)
-        return fail(TFRPN_ERR_UNSUPPORTED, "NMS: %d output rows need %zu B of shared memory (> %zu)", p.max_out, smem,
-                    PROP_SMEM_LIMIT);
+    if (int rc = check_prop_smem(smem, p.max_out)) return rc;
     threads = h->opts.prop_threads;
     if (threads != 512 && threads != 1024) {
         int per_sm = 0;
@@ -2616,10 +2523,7 @@ extern "C" int tfrpn_nms_multiclass(tfrpn_handle h, const float* boxes, int q, c
     {   // the per-class kernel's shared-memory carve bounds max_output_size_per_class, as in tfrpn_nms
         int cl = 0, threads = 1024;
         pick_cluster(h, S, cl, threads);
-        const size_t smem = cl ? cluster_smem_bytes(cl, 0, P) : prop_smem_bytes(0, P);
-        if (smem > PROP_SMEM_LIMIT)
-            return fail(TFRPN_ERR_UNSUPPORTED, "NMS: %d output rows need %zu B of shared memory (> %zu)", P, smem,
-                        PROP_SMEM_LIMIT);
+        if (int rc = check_prop_smem(cl ? cluster_smem_bytes(cl, 0, P) : prop_smem_bytes(0, P), P)) return rc;
     }
     McLayout L;
     mc_layout(B, K, C, cfg, &L, h->opts.nms_mc_stage);
