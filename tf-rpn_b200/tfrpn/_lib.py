@@ -97,6 +97,8 @@ PROTOTYPES = {
     "tfrpn_rpn_targets_compact": (I, [P, P, P, P, I, I, I, C.POINTER(TargetCfg), P, P, P, P]),
     "tfrpn_expand_targets_host": (I, [P, P, I, I, I, P, I, P]),
     "tfrpn_roi_targets": (I, [P, P, P, P, P, I, I, I, C.POINTER(RoiTargetCfg), P, P, P, P, P, P, P, P]),
+    "tfrpn_crop_and_resize": (I, [P, I, I, I, I, P, P, I, I, I, C.c_float, P, P]),
+    "tfrpn_crop_and_resize_grad_image": (I, [P, P, P, I, I, I, I, I, I, I, P, P]),
     "tfrpn_select_mask": (I, [P, P, P, I, I, I, C.c_uint64, C.c_uint64, I, I, P, P]),
     "tfrpn_rpn_losses": (I, [P, P, P, P, P, I, I, C.c_float, P, P, P, P]),
     "tfrpn_topk": (I, [P, P, I, I, I, P, P, P, I, P, P]),
