@@ -271,6 +271,256 @@ size_t losses_workspace_bytes(long long total) {
     return (size_t)((total + LOSS_THREADS * LOSS_EPT - 1) / (LOSS_THREADS * LOSS_EPT) + 1) * sizeof(LossPartial) + 256;
 }
 
+// ---- the second stage's box-head losses (tfrpn_roi_head_losses) ------------------------------------------------------
+//   L1 roi_loss_partial_kernel<G>  a group of G lanes per row: the lanes stride over the row's logits in chunks of 4
+//                                  classes (lane g takes chunks g, g + G, ...; a float4 load where the row is 16-byte
+//                                  aligned, 4 scalar loads otherwise: the same values in the same order) for the max,
+//                                  then the exp-sum and the argmax; lane 0 of the group adds the row's terms.  The box
+//                                  deltas are read for fg rows only, 16 bytes per row.  The sums and counts go through
+//                                  the partial / last-CTA scheme of rpn_loss_partial_kernel (ticket word 1).
+//   L2 roi_loss_grad_kernel<G>     recomputes each row's max and exp-sum with the same code, so e_c / s has the bits
+//                                  L1 saw, and writes both gradients everywhere, scaled by the counts L1 left in out.
+// G (4, 8, 16 or 32) is the smallest that covers the ceil(C / 4) chunks, 32 above: C = 21 takes 8 lanes per row, C = 81
+// takes 32.  The grid is capped at a constant, so the partition of the sums depends on the shape alone.
+constexpr int ROI_LOSS_MAX_CTAS = 1184;   // 8 CTAs of 256 threads on each of 148 SMs
+
+struct RoiLossPartial {
+    float4 sums;    // cls.hi, cls.lo, reg.hi, reg.lo
+    uint4 counts;   // n_rows, n_fg, n_correct, n_fg_correct
+};
+
+template <int G>
+__device__ __forceinline__ float group_max(float v) {
+#pragma unroll
+    for (int o = G / 2; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
+    return v;
+}
+template <int G>
+__device__ __forceinline__ float group_sum(float v) {   // a butterfly: every lane of the group gets the same bits
+#pragma unroll
+    for (int o = G / 2; o > 0; o >>= 1) v = __fadd_rn(v, __shfl_xor_sync(0xffffffffu, v, o));
+    return v;
+}
+template <int G>
+__device__ __forceinline__ int group_min(int v) {
+#pragma unroll
+    for (int o = G / 2; o > 0; o >>= 1) v = min(v, __shfl_xor_sync(0xffffffffu, v, o));
+    return v;
+}
+
+// classes c0 .. c0 + 3 of a row (those < C); vec: C % 4 == 0 and the row is 16-byte aligned
+__device__ __forceinline__ void load_chunk(const float* __restrict__ x, int c0, int C, bool vec, float v[4]) {
+    if (vec) {
+        const float4 q = __ldg(reinterpret_cast<const float4*>(x + c0));
+        v[0] = q.x; v[1] = q.y; v[2] = q.z; v[3] = q.w;
+        return;
+    }
+#pragma unroll
+    for (int j = 0; j < 4; ++j) v[j] = c0 + j < C ? __ldg(x + c0 + j) : 0.0f;
+}
+
+// One row's softmax statistics, the same on every lane of the group: m = max (NaN ignored), s = sum of
+// expf(x_c - m) (NaN when any logit is NaN), first = the first c with x_c == m, nan = any logit is NaN.  C_eff = 0
+// (a row that takes no part) reads nothing but keeps the group in step with the shuffles.
+template <int G>
+__device__ __forceinline__ void roi_row_stats(const float* __restrict__ x, int C_eff, bool vec, int g, float& m,
+                                              float& s, int& first, bool& nan) {
+    float mx = -INFINITY;
+    bool bad = false;
+    for (int c0 = 4 * g; c0 < C_eff; c0 += 4 * G) {
+        float v[4];
+        load_chunk(x, c0, C_eff, vec, v);
+#pragma unroll
+        for (int j = 0; j < 4; ++j)
+            if (c0 + j < C_eff) { bad |= isnan(v[j]); mx = fmaxf(mx, v[j]); }
+    }
+    m = group_max<G>(mx);
+    nan = group_min<G>(bad ? 0 : 1) == 0;
+    float sum = 0.0f;
+    int arg = C_eff;
+    for (int c0 = 4 * g; c0 < C_eff; c0 += 4 * G) {
+        float v[4];
+        load_chunk(x, c0, C_eff, vec, v);
+#pragma unroll
+        for (int j = 0; j < 4; ++j)
+            if (c0 + j < C_eff) {
+                sum = __fadd_rn(sum, expf(__fsub_rn(v[j], m)));
+                if (v[j] == m && arg == C_eff) arg = c0 + j;
+            }
+    }
+    s = group_sum<G>(sum);
+    first = group_min<G>(arg);
+}
+
+__device__ __forceinline__ float huber_row(float4 t, float4 p, float delta) {   // reduce_sum over the 4 coordinates
+    float row = huber_term(t.x, p.x, delta);
+    row = __fadd_rn(row, huber_term(t.y, p.y, delta));
+    row = __fadd_rn(row, huber_term(t.z, p.z, delta));
+    return __fadd_rn(row, huber_term(t.w, p.w, delta));
+}
+
+template <int G>
+__global__ void __launch_bounds__(LOSS_THREADS) roi_loss_partial_kernel(
+    const float* __restrict__ logits, const float4* __restrict__ box_deltas, const int* __restrict__ labels,
+    const float4* __restrict__ targets, long long rows, int C, int q, float delta, int norm_rows, bool vec,
+    RoiLossPartial* __restrict__ partials, unsigned int* __restrict__ ticket, tfrpn_roi_loss_out* __restrict__ out) {
+    constexpr int RPW = 32 / G;   // rows per warp and pass
+    const int g = lane_id() % G;
+    float2 cls = make_float2(0.f, 0.f), reg = make_float2(0.f, 0.f);
+    unsigned n_rows = 0u, n_fg = 0u, n_ok = 0u, n_fg_ok = 0u;
+    const long long stride = (long long)gridDim.x * (LOSS_THREADS / 32) * RPW;
+    for (long long r0 = ((long long)blockIdx.x * (LOSS_THREADS / 32) + warp_id()) * RPW; r0 < rows; r0 += stride) {
+        const long long r = r0 + lane_id() / G;
+        const int label = r < rows ? __ldg(labels + r) : -1;
+        const bool part = label >= 0 && label < C;
+        const float* x = logits + (part ? r : 0) * C;
+        float m, s;
+        int first;
+        bool nan;
+        roi_row_stats<G>(x, part ? C : 0, vec, g, m, s, first, nan);
+        if (part && g == 0) {
+            const float term = __fsub_rn(logf(s), __fsub_rn(__ldg(x + label), m));
+            const unsigned ok = (!nan && first == label) ? 1u : 0u;
+            cls = pair_add(cls, make_float2(term, 0.0f));
+            ++n_rows;
+            n_ok += ok;
+            if (label >= 1) {
+                const float4 t = ldg_f4(targets + r);
+                const float4 p = ldg_f4(box_deltas + r * q + (q == C ? label : 0));
+                reg = pair_add(reg, make_float2(huber_row(t, p, delta), 0.0f));
+                ++n_fg;
+                n_fg_ok += ok;
+            }
+        }
+    }
+    __shared__ float2 s_cls[LOSS_THREADS / 32], s_reg[LOSS_THREADS / 32];
+    __shared__ uint4 s_n[LOSS_THREADS / 32];
+    __shared__ bool s_last;
+    const float2 cls2 = warp_pair_sum(cls.x), cls2lo = warp_pair_sum(cls.y);
+    const float2 reg2 = warp_pair_sum(reg.x), reg2lo = warp_pair_sum(reg.y);
+    const uint4 n = make_uint4(warp_sum(n_rows), warp_sum(n_fg), warp_sum(n_ok), warp_sum(n_fg_ok));
+    if (lane_id() == 0) {
+        s_cls[warp_id()] = pair_add(cls2, cls2lo);
+        s_reg[warp_id()] = pair_add(reg2, reg2lo);
+        s_n[warp_id()] = n;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float2 c = s_cls[0], rg = s_reg[0];
+        uint4 k = s_n[0];
+        for (int w = 1; w < LOSS_THREADS / 32; ++w) {
+            c = pair_add(c, s_cls[w]);
+            rg = pair_add(rg, s_reg[w]);
+            k.x += s_n[w].x; k.y += s_n[w].y; k.z += s_n[w].z; k.w += s_n[w].w;
+        }
+        RoiLossPartial p;
+        p.sums = make_float4(c.x, c.y, rg.x, rg.y);
+        p.counts = k;
+        partials[blockIdx.x] = p;
+        __threadfence();
+        s_last = atomicAdd(ticket, 1u) == gridDim.x - 1;
+    }
+    __syncthreads();
+    if (!s_last) return;
+    // the last CTA: the partials in a fixed order (grid <= ROI_LOSS_MAX_CTAS, so one warp walks them), then doubles
+    __threadfence();
+    if (threadIdx.x >= 32) return;
+    float2 c2 = make_float2(0.f, 0.f), r2 = make_float2(0.f, 0.f);
+    unsigned long long k2[4] = {0ull, 0ull, 0ull, 0ull};
+    for (int i = lane_id(); i < (int)gridDim.x; i += 32) {
+        const float4 v = __ldcg(&partials[i].sums);
+        const uint4 k = __ldcg(&partials[i].counts);
+        c2 = pair_add(c2, make_float2(v.x, v.y));
+        r2 = pair_add(r2, make_float2(v.z, v.w));
+        k2[0] += k.x; k2[1] += k.y; k2[2] += k.z; k2[3] += k.w;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        float2 t;
+        t.x = __shfl_xor_sync(0xffffffffu, c2.x, o); t.y = __shfl_xor_sync(0xffffffffu, c2.y, o);
+        c2 = pair_add(c2, t);
+        t.x = __shfl_xor_sync(0xffffffffu, r2.x, o); t.y = __shfl_xor_sync(0xffffffffu, r2.y, o);
+        r2 = pair_add(r2, t);
+#pragma unroll
+        for (int j = 0; j < 4; ++j) k2[j] += __shfl_xor_sync(0xffffffffu, k2[j], o);
+    }
+    if (lane_id() == 0) {
+        const double Cs = (double)c2.x + (double)c2.y, R = (double)r2.x + (double)r2.y;
+        const unsigned long long norm = norm_rows ? k2[0] : k2[1];
+        tfrpn_roi_loss_out res;
+        res.cls_loss = (float)(Cs / (double)k2[0]);                      // 0/0 -> NaN
+        res.reg_loss = (float)(R / (double)(norm > 0ull ? norm : 1ull));
+        res.n_rows = (int32_t)k2[0];
+        res.n_fg = (int32_t)k2[1];
+        res.n_correct = (int32_t)k2[2];
+        res.n_fg_correct = (int32_t)k2[3];
+        res.reserved[0] = res.reserved[1] = 0;
+        *out = res;
+        *ticket = 0u;     // ready for the next call on this handle
+    }
+}
+
+template <int G>
+__global__ void __launch_bounds__(LOSS_THREADS) roi_loss_grad_kernel(
+    const float* __restrict__ logits, const float4* __restrict__ box_deltas, const int* __restrict__ labels,
+    const float4* __restrict__ targets, long long rows, int C, int q, float delta, int norm_rows, bool vec_in,
+    bool vec_out, const tfrpn_roi_loss_out* __restrict__ res, const float* __restrict__ scale,
+    float* __restrict__ grad_logits, float4* __restrict__ grad_deltas) {
+    constexpr int RPW = 32 / G;
+    const int g = lane_id() % G;
+    const int n_rows = res->n_rows;
+    const float inv_rows = __fdiv_rn(1.0f, (float)n_rows);
+    const float inv_reg = __fdiv_rn(1.0f, (float)max(norm_rows ? n_rows : res->n_fg, 1));
+    const float s_cls = scale ? scale[0] : 1.0f, s_reg = scale ? scale[1] : 1.0f;
+    const long long stride = (long long)gridDim.x * (LOSS_THREADS / 32) * RPW;
+    for (long long r0 = ((long long)blockIdx.x * (LOSS_THREADS / 32) + warp_id()) * RPW; r0 < rows; r0 += stride) {
+        const long long r = r0 + lane_id() / G;
+        const bool in = r < rows;
+        const int label = in ? __ldg(labels + r) : -1;
+        const bool part = label >= 0 && label < C;
+        if (grad_logits) {
+            const float* x = logits + (part ? r : 0) * C;
+            float m, s;
+            int first;
+            bool nan;
+            roi_row_stats<G>(x, part ? C : 0, vec_in, g, m, s, first, nan);
+            float* gx = grad_logits + (in ? r : 0) * C;
+            for (int c0 = 4 * g; in && c0 < C; c0 += 4 * G) {
+                float v[4] = {0.f, 0.f, 0.f, 0.f};
+                if (part) {
+                    load_chunk(x, c0, C, vec_in, v);
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) {
+                        const float p = __fdiv_rn(expf(__fsub_rn(v[j], m)), s);
+                        v[j] = __fmul_rn(__fmul_rn(__fsub_rn(p, c0 + j == label ? 1.0f : 0.0f), inv_rows), s_cls);
+                    }
+                }
+                if (vec_out) {
+                    stg_f4_stream(reinterpret_cast<float4*>(gx + c0), make_float4(v[0], v[1], v[2], v[3]));
+                } else {
+#pragma unroll
+                    for (int j = 0; j < 4; ++j)
+                        if (c0 + j < C) stg_f1_stream(gx + c0 + j, v[j]);
+                }
+            }
+        }
+        if (grad_deltas && in) {
+            float4 gsel = make_float4(0.f, 0.f, 0.f, 0.f);
+            int sel = -1;
+            if (label >= 1 && label < C) {
+                sel = q == C ? label : 0;
+                const float4 t = ldg_f4(targets + r), p = ldg_f4(box_deltas + r * q + sel);
+                gsel = make_float4(__fmul_rn(__fmul_rn(huber_grad(t.x, p.x, delta), inv_reg), s_reg),
+                                   __fmul_rn(__fmul_rn(huber_grad(t.y, p.y, delta), inv_reg), s_reg),
+                                   __fmul_rn(__fmul_rn(huber_grad(t.z, p.z, delta), inv_reg), s_reg),
+                                   __fmul_rn(__fmul_rn(huber_grad(t.w, p.w, delta), inv_reg), s_reg));
+            }
+            for (int k = g; k < q; k += G)
+                stg_f4_stream(grad_deltas + r * q + k, k == sel ? gsel : make_float4(0.f, 0.f, 0.f, 0.f));
+        }
+    }
+}
+
 }  // namespace tfrpn
 
 using namespace tfrpn;
@@ -316,4 +566,79 @@ extern "C" int tfrpn_rpn_losses(tfrpn_handle h, const float* true_deltas, const 
         TFRPN_AFTER_LAUNCH("rpn_loss_grad_kernel");
     }
     return 0;
+}
+
+namespace {
+long long roi_loss_ctas(long long rows, int G) {
+    const long long per_cta = (LOSS_THREADS / 32) * (32 / G);
+    return std::max(1LL, std::min((rows + per_cta - 1) / per_cta, (long long)ROI_LOSS_MAX_CTAS));
+}
+
+template <int G>
+int launch_roi_losses(const float* logits, const float4* bd, const int32_t* labels, const float4* td, long long rows,
+                      const tfrpn_roi_loss_cfg& cfg, char* ws, unsigned int* ticket, tfrpn_roi_loss_out* out,
+                      const float* scale, float* grad_logits, float4* grad_deltas, cudaStream_t st) {
+    const int C = cfg.num_classes, q = cfg.box_classes;
+    const int ctas = (int)roi_loss_ctas(rows, G);
+    const bool vec_in = C % 4 == 0 && aligned16(logits);
+    roi_loss_partial_kernel<G><<<ctas, LOSS_THREADS, 0, st>>>(logits, bd, labels, td, rows, C, q, cfg.huber_delta,
+                                                              cfg.reg_normalizer, vec_in,
+                                                              reinterpret_cast<RoiLossPartial*>(ws), ticket, out);
+    TFRPN_AFTER_LAUNCH("roi_loss_partial_kernel");
+    if ((grad_logits || grad_deltas) && rows > 0) {
+        const bool vec_out = C % 4 == 0 && aligned16(grad_logits);
+        roi_loss_grad_kernel<G><<<ctas, LOSS_THREADS, 0, st>>>(logits, bd, labels, td, rows, C, q, cfg.huber_delta,
+                                                               cfg.reg_normalizer, vec_in, vec_out, out, scale,
+                                                               grad_logits, grad_deltas);
+        TFRPN_AFTER_LAUNCH("roi_loss_grad_kernel");
+    }
+    return 0;
+}
+}  // namespace
+
+extern "C" int tfrpn_roi_head_losses(tfrpn_handle h, const float* cls_logits, const float* box_deltas,
+                                     const int32_t* labels, const float* target_deltas, int B, int S,
+                                     const tfrpn_roi_loss_cfg* cfg, tfrpn_roi_loss_out* out,
+                                     const float* grad_scale_or_null, float* grad_logits_or_null,
+                                     float* grad_deltas_or_null, tfrpn_stream s) {
+    if (!h) return fail(TFRPN_ERR_BAD_ARG, "roi_head_losses: null handle");
+    if (!cls_logits || !box_deltas || !labels || !target_deltas || !cfg || !out)
+        return fail(TFRPN_ERR_BAD_ARG, "roi_head_losses: null cls_logits, box_deltas, labels, target_deltas, cfg or out");
+    if (B < 0 || S < 0) return fail(TFRPN_ERR_BAD_ARG, "roi_head_losses: negative shape");
+    const int C = cfg->num_classes, q = cfg->box_classes;
+    if (C < 2) return fail(TFRPN_ERR_BAD_ARG, "roi_head_losses: num_classes must be >= 2, got %d", C);
+    if (q != 1 && q != C) return fail(TFRPN_ERR_BAD_ARG, "roi_head_losses: box_classes must be 1 or %d, got %d", C, q);
+    if (!(cfg->huber_delta > 0.0f)) return fail(TFRPN_ERR_BAD_ARG, "roi_head_losses: huber_delta must be > 0");
+    if (cfg->reg_normalizer != 0 && cfg->reg_normalizer != 1)
+        return fail(TFRPN_ERR_BAD_ARG, "roi_head_losses: reg_normalizer must be 0 or 1, got %d", cfg->reg_normalizer);
+    if (C > 1024 || S > 8192 || B > 65535)
+        return fail(TFRPN_ERR_UNSUPPORTED, "roi_head_losses: C = %d, S = %d, B = %d beyond 1024, 8192, 65535", C, S, B);
+    if (!aligned16(box_deltas) || !aligned16(target_deltas) || (grad_deltas_or_null && !aligned16(grad_deltas_or_null)))
+        return fail(TFRPN_ERR_MISALIGNED, "roi_head_losses: box_deltas, target_deltas and grad_deltas must be 16-byte aligned");
+    const auto a4 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 3u) == 0; };
+    if (!a4(cls_logits) || !a4(labels) || !a4(grad_logits_or_null))
+        return fail(TFRPN_ERR_MISALIGNED, "roi_head_losses: cls_logits, labels and grad_logits must be 4-byte aligned");
+    TFRPN_ENTER(h);
+    TFRPN_CHECK_ON_DEVICE(h, out, "roi_head_losses: out");
+    TFRPN_CHECK_ON_DEVICE(h, cls_logits, "roi_head_losses: cls_logits");
+    cudaStream_t st = as_stream(s);
+    const long long rows = (long long)B * S;
+    const int G = (C + 3) / 4 <= 4 ? 4 : (C + 3) / 4 <= 8 ? 8 : (C + 3) / 4 <= 16 ? 16 : 32;
+    char* ws = nullptr;
+    if (int rc = ensure_workspace(h, (size_t)roi_loss_ctas(rows, G) * sizeof(RoiLossPartial) + 256, st, &ws)) return rc;
+    if (!h->ticket) return fail(TFRPN_ERR_CUDA, "roi_head_losses: the handle has no device counter");
+    const float4* bd = reinterpret_cast<const float4*>(box_deltas);
+    const float4* td = reinterpret_cast<const float4*>(target_deltas);
+    float4* gd = reinterpret_cast<float4*>(grad_deltas_or_null);
+    unsigned int* ticket = h->ticket + 1;
+    switch (G) {
+        case 4: return launch_roi_losses<4>(cls_logits, bd, labels, td, rows, *cfg, ws, ticket, out, grad_scale_or_null,
+                                            grad_logits_or_null, gd, st);
+        case 8: return launch_roi_losses<8>(cls_logits, bd, labels, td, rows, *cfg, ws, ticket, out, grad_scale_or_null,
+                                            grad_logits_or_null, gd, st);
+        case 16: return launch_roi_losses<16>(cls_logits, bd, labels, td, rows, *cfg, ws, ticket, out, grad_scale_or_null,
+                                              grad_logits_or_null, gd, st);
+        default: return launch_roi_losses<32>(cls_logits, bd, labels, td, rows, *cfg, ws, ticket, out, grad_scale_or_null,
+                                              grad_logits_or_null, gd, st);
+    }
 }

@@ -65,6 +65,16 @@ class RoiTargetCfg(C.Structure):
                 ("seed", C.c_uint64), ("offset", C.c_uint64)]
 
 
+class RoiLossCfg(C.Structure):
+    _fields_ = [("num_classes", C.c_int32), ("box_classes", C.c_int32), ("huber_delta", C.c_float),
+                ("reg_normalizer", C.c_int32)]
+
+
+class RoiLossOut(C.Structure):
+    _fields_ = [("cls_loss", C.c_float), ("reg_loss", C.c_float), ("n_rows", C.c_int32), ("n_fg", C.c_int32),
+                ("n_correct", C.c_int32), ("n_fg_correct", C.c_int32), ("reserved", C.c_int32 * 2)]
+
+
 class StepBuffers(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("gt_boxes", "gt_labels", "rpn_reg", "rpn_cls", "deltas", "labels",
                                           "out_boxes", "out_scores", "valid", "keep_idx")]
@@ -97,6 +107,7 @@ PROTOTYPES = {
     "tfrpn_rpn_targets_compact": (I, [P, P, P, P, I, I, I, C.POINTER(TargetCfg), P, P, P, P]),
     "tfrpn_expand_targets_host": (I, [P, P, I, I, I, P, I, P]),
     "tfrpn_roi_targets": (I, [P, P, P, P, P, I, I, I, C.POINTER(RoiTargetCfg), P, P, P, P, P, P, P, P]),
+    "tfrpn_roi_head_losses": (I, [P, P, P, P, P, I, I, C.POINTER(RoiLossCfg), P, P, P, P, P]),
     "tfrpn_crop_and_resize": (I, [P, I, I, I, I, P, P, I, I, I, C.c_float, P, P]),
     "tfrpn_crop_and_resize_grad_image": (I, [P, P, P, I, I, I, I, I, I, I, P, P]),
     "tfrpn_select_mask": (I, [P, P, P, I, I, I, C.c_uint64, C.c_uint64, I, I, P, P]),
