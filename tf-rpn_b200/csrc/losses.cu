@@ -13,7 +13,7 @@
 //                               warp, doubles above), one partial per CTA; the last CTA
 //                               sums the partials in a fixed order (deterministic) and divides.
 //   L2 rpn_loss_grad_kernel     elementwise gradients, scaled by the counts L1 left on the device.
-#include "common.cuh"
+#include "roi_rows.cuh"
 
 namespace tfrpn {
 
@@ -289,69 +289,6 @@ struct RoiLossPartial {
     uint4 counts;   // n_rows, n_fg, n_correct, n_fg_correct
 };
 
-template <int G>
-__device__ __forceinline__ float group_max(float v) {
-#pragma unroll
-    for (int o = G / 2; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-    return v;
-}
-template <int G>
-__device__ __forceinline__ float group_sum(float v) {   // a butterfly: every lane of the group gets the same bits
-#pragma unroll
-    for (int o = G / 2; o > 0; o >>= 1) v = __fadd_rn(v, __shfl_xor_sync(0xffffffffu, v, o));
-    return v;
-}
-template <int G>
-__device__ __forceinline__ int group_min(int v) {
-#pragma unroll
-    for (int o = G / 2; o > 0; o >>= 1) v = min(v, __shfl_xor_sync(0xffffffffu, v, o));
-    return v;
-}
-
-// classes c0 .. c0 + 3 of a row (those < C); vec: C % 4 == 0 and the row is 16-byte aligned
-__device__ __forceinline__ void load_chunk(const float* __restrict__ x, int c0, int C, bool vec, float v[4]) {
-    if (vec) {
-        const float4 q = __ldg(reinterpret_cast<const float4*>(x + c0));
-        v[0] = q.x; v[1] = q.y; v[2] = q.z; v[3] = q.w;
-        return;
-    }
-#pragma unroll
-    for (int j = 0; j < 4; ++j) v[j] = c0 + j < C ? __ldg(x + c0 + j) : 0.0f;
-}
-
-// One row's softmax statistics, the same on every lane of the group: m = max (NaN ignored), s = sum of
-// expf(x_c - m) (NaN when any logit is NaN), first = the first c with x_c == m, nan = any logit is NaN.  C_eff = 0
-// (a row that takes no part) reads nothing but keeps the group in step with the shuffles.
-template <int G>
-__device__ __forceinline__ void roi_row_stats(const float* __restrict__ x, int C_eff, bool vec, int g, float& m,
-                                              float& s, int& first, bool& nan) {
-    float mx = -INFINITY;
-    bool bad = false;
-    for (int c0 = 4 * g; c0 < C_eff; c0 += 4 * G) {
-        float v[4];
-        load_chunk(x, c0, C_eff, vec, v);
-#pragma unroll
-        for (int j = 0; j < 4; ++j)
-            if (c0 + j < C_eff) { bad |= isnan(v[j]); mx = fmaxf(mx, v[j]); }
-    }
-    m = group_max<G>(mx);
-    nan = group_min<G>(bad ? 0 : 1) == 0;
-    float sum = 0.0f;
-    int arg = C_eff;
-    for (int c0 = 4 * g; c0 < C_eff; c0 += 4 * G) {
-        float v[4];
-        load_chunk(x, c0, C_eff, vec, v);
-#pragma unroll
-        for (int j = 0; j < 4; ++j)
-            if (c0 + j < C_eff) {
-                sum = __fadd_rn(sum, expf(__fsub_rn(v[j], m)));
-                if (v[j] == m && arg == C_eff) arg = c0 + j;
-            }
-    }
-    s = group_sum<G>(sum);
-    first = group_min<G>(arg);
-}
-
 __device__ __forceinline__ float huber_row(float4 t, float4 p, float delta) {   // reduce_sum over the 4 coordinates
     float row = huber_term(t.x, p.x, delta);
     row = __fadd_rn(row, huber_term(t.y, p.y, delta));
@@ -623,7 +560,7 @@ extern "C" int tfrpn_roi_head_losses(tfrpn_handle h, const float* cls_logits, co
     TFRPN_CHECK_ON_DEVICE(h, cls_logits, "roi_head_losses: cls_logits");
     cudaStream_t st = as_stream(s);
     const long long rows = (long long)B * S;
-    const int G = (C + 3) / 4 <= 4 ? 4 : (C + 3) / 4 <= 8 ? 8 : (C + 3) / 4 <= 16 ? 16 : 32;
+    const int G = roi_row_lanes(C);
     char* ws = nullptr;
     if (int rc = ensure_workspace(h, (size_t)roi_loss_ctas(rows, G) * sizeof(RoiLossPartial) + 256, st, &ws)) return rc;
     if (!h->ticket) return fail(TFRPN_ERR_CUDA, "roi_head_losses: the handle has no device counter");

@@ -2454,9 +2454,12 @@ static bool mc_rows_apply(int mode, int B, int K, int C) {
     if (C > MC_ROW_MAX_C || (long long)K * C > 0x7FFFFFFFLL || mode == 1) return false;
     return mode == 2 || (long long)B * C < 148;
 }
-static void mc_layout(int B, int K, int C, const tfrpn_nms_cfg* cfg, McLayout* L, int stage_mode = 0) {
+// row_classes: the classes of the output-row rule (C; C - 1 for the box-head detections, whose class 0 never has a
+// candidate).  The sizes do not depend on it: lmax = min(P, total) for any row_classes >= 1.
+static void mc_layout(int B, int K, int C, const tfrpn_nms_cfg* cfg, McLayout* L, int stage_mode = 0, int row_classes = 0) {
     const int P = cfg->max_output_size_per_class;
-    L->rows = cfg->pad_per_class ? (int)std::min((long long)cfg->max_total_size, (long long)P * C) : cfg->max_total_size;
+    const long long rc = row_classes > 0 ? row_classes : C;
+    L->rows = cfg->pad_per_class ? (int)std::min((long long)cfg->max_total_size, (long long)P * rc) : cfg->max_total_size;
     L->lmax = min(P, L->rows);
     L->scratch = ((long long)C * 16 + (long long)C * L->lmax * 4 + 15) & ~15LL;
     // ~2 CTAs per SM over the batch, no more than there are slices of MC_MERGE_THREADS entries
@@ -2480,7 +2483,7 @@ static void mc_layout(int B, int K, int C, const tfrpn_nms_cfg* cfg, McLayout* L
     L->row_cnt = o;     o += align256((size_t)B * L->slices * MC_ROW_WARPS * C * 4);   // (counted in every mode)
     L->total = o + 256;
 }
-static int mc_check_sizes(const char* fn, int B, int K, int C, const tfrpn_nms_cfg* cfg) {
+int mc_check_sizes(const char* fn, int B, int K, int C, const tfrpn_nms_cfg* cfg) {
     if (!cfg) return fail(TFRPN_ERR_BAD_ARG, "%s: null cfg", fn);
     if (B <= 0 || K <= 0 || C < 1) return fail(TFRPN_ERR_BAD_ARG, "%s: B=%d, K=%d, C=%d must be > 0", fn, B, K, C);
     if ((long long)B * C > 0x7FFFFFFFLL) return fail(TFRPN_ERR_BAD_ARG, "%s: B * C = %lld segments", fn, (long long)B * C);
@@ -2506,33 +2509,32 @@ extern "C" int tfrpn_reserve_nms_multiclass(tfrpn_handle h, int B, int K, int C,
     return ensure_workspace_prop(h, tfrpn_nms_multiclass_workspace_bytes(B, K, C, cfg), nullptr, &ws);
 }
 
-extern "C" int tfrpn_nms_multiclass(tfrpn_handle h, const float* boxes, int q, const float* scores, int B, int K, int C,
-                                    const tfrpn_nms_cfg* cfg, float* out_boxes, float* out_scores, float* out_classes,
-                                    int32_t* valid, int32_t* keep_idx_or_null, tfrpn_stream s) {
-    if (!boxes || !scores || !cfg || !out_boxes || !out_scores || !out_classes || !valid)
-        return fail(TFRPN_ERR_BAD_ARG, "nms_multiclass: null pointer");
-    if (int rc = mc_check_sizes("nms_multiclass", B, K, C, cfg)) return rc;
-    if (q != 1 && q != C) return fail(TFRPN_ERR_BAD_ARG, "nms_multiclass: q = %d must be 1 or C = %d", q, C);
-    if (!aligned16(boxes) || !aligned16(out_boxes))
-        return fail(TFRPN_ERR_MISALIGNED, "nms_multiclass: boxes must be 16-byte aligned");
-    if (!h) return fail(TFRPN_ERR_BAD_ARG, "nms_multiclass: null handle");
-    TFRPN_ENTER(h);
-    TFRPN_CHECK_ON_DEVICE(h, boxes, "nms_multiclass: boxes");
-    cudaStream_t st = as_stream(s);
+namespace tfrpn {
+// the per-class kernel's shared-memory carve bounds max_output_size_per_class, as in tfrpn_nms
+int nms_mc_check_smem(tfrpn_handle h, int B, int C, int P) {
+    int cl = 0, threads = 1024;
+    pick_cluster(h, B * C, cl, threads);
+    return check_prop_smem(cl ? cluster_smem_bytes(cl, 0, P) : prop_smem_bytes(0, P), P);
+}
+
+// The body of tfrpn_nms_multiclass after its argument checks, shared with tfrpn_roi_head_detections (roi_detect.cu).
+// Candidates are the entries with score > sthr (use_sthr) or all of them; output rows follow the rule with
+// row_classes classes.  The layout starts ws_offset bytes into the proposal-side workspace: the bytes before it are
+// the caller's (the detections' staged scores and boxes, written before this call).
+int nms_mc_run(tfrpn_handle h, const float* boxes, int q, const float* scores, int B, int K, int C,
+               const tfrpn_nms_cfg* cfg, int row_classes, int use_sthr, float sthr, size_t ws_offset, float* out_boxes,
+               float* out_scores, float* out_classes, int32_t* valid, int32_t* keep_idx_or_null, cudaStream_t st) {
     const int S = B * C, P = cfg->max_output_size_per_class;
-    {   // the per-class kernel's shared-memory carve bounds max_output_size_per_class, as in tfrpn_nms
-        int cl = 0, threads = 1024;
-        pick_cluster(h, S, cl, threads);
-        if (int rc = check_prop_smem(cl ? cluster_smem_bytes(cl, 0, P) : prop_smem_bytes(0, P), P)) return rc;
-    }
+    if (int rc = nms_mc_check_smem(h, B, C, P)) return rc;
     McLayout L;
-    mc_layout(B, K, C, cfg, &L, h->opts.nms_mc_stage);
+    mc_layout(B, K, C, cfg, &L, h->opts.nms_mc_stage, row_classes);
     char* ws = nullptr;
-    if (int rc = ensure_workspace_prop(h, L.total, st, &ws)) return rc;
+    if (int rc = ensure_workspace_prop(h, ws_offset + L.total, st, &ws)) return rc;
+    ws += ws_offset;
 
     McStageParams g = {};
     g.scores = scores; g.boxes = reinterpret_cast<const float4*>(boxes); g.K = K; g.C = C; g.q = q;
-    g.use_sthr = !(cfg->score_threshold == -INFINITY); g.sthr = cfg->score_threshold;
+    g.use_sthr = use_sthr; g.sthr = sthr;
     g.cand_scores = reinterpret_cast<float*>(ws + L.cand_scores); g.remap = reinterpret_cast<int*>(ws + L.remap);
     g.cand_boxes = reinterpret_cast<float4*>(ws + L.cand_boxes); g.counts = reinterpret_cast<int*>(ws + L.counts);
     prof_begin(h, TFRPN_K_NMS_MC_STAGE, st);
@@ -2572,6 +2574,23 @@ extern "C" int tfrpn_nms_multiclass(tfrpn_handle h, const float* boxes, int q, c
     prof_end(h, st);
     TFRPN_AFTER_LAUNCH("nms_mc_merge_kernel");
     return 0;
+}
+}  // namespace tfrpn
+
+extern "C" int tfrpn_nms_multiclass(tfrpn_handle h, const float* boxes, int q, const float* scores, int B, int K, int C,
+                                    const tfrpn_nms_cfg* cfg, float* out_boxes, float* out_scores, float* out_classes,
+                                    int32_t* valid, int32_t* keep_idx_or_null, tfrpn_stream s) {
+    if (!boxes || !scores || !cfg || !out_boxes || !out_scores || !out_classes || !valid)
+        return fail(TFRPN_ERR_BAD_ARG, "nms_multiclass: null pointer");
+    if (int rc = mc_check_sizes("nms_multiclass", B, K, C, cfg)) return rc;
+    if (q != 1 && q != C) return fail(TFRPN_ERR_BAD_ARG, "nms_multiclass: q = %d must be 1 or C = %d", q, C);
+    if (!aligned16(boxes) || !aligned16(out_boxes))
+        return fail(TFRPN_ERR_MISALIGNED, "nms_multiclass: boxes must be 16-byte aligned");
+    if (!h) return fail(TFRPN_ERR_BAD_ARG, "nms_multiclass: null handle");
+    TFRPN_ENTER(h);
+    TFRPN_CHECK_ON_DEVICE(h, boxes, "nms_multiclass: boxes");
+    return nms_mc_run(h, boxes, q, scores, B, K, C, cfg, C, !(cfg->score_threshold == -INFINITY), cfg->score_threshold, 0,
+                      out_boxes, out_scores, out_classes, valid, keep_idx_or_null, as_stream(s));
 }
 
 #ifdef TFRPN_PHASE_TIMING

@@ -13,5 +13,6 @@ from .evaluation import DetectionMAP, ProposalRecall, detection_map, proposal_re
 from .roi_targets import RoiTargets, roi_target_cfg, roi_targets  # noqa: F401
 from .roi_crop import crop_and_resize  # noqa: F401
 from .roi_losses import RoiHeadLosses, roi_head_losses  # noqa: F401
+from .roi_detections import roi_head_detections  # noqa: F401
 
 __version__ = "0.1.0"

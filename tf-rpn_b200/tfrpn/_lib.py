@@ -75,6 +75,12 @@ class RoiLossOut(C.Structure):
                 ("n_correct", C.c_int32), ("n_fg_correct", C.c_int32), ("reserved", C.c_int32 * 2)]
 
 
+class RoiDetCfg(C.Structure):
+    _fields_ = [("num_classes", C.c_int32), ("box_classes", C.c_int32), ("score_input", C.c_int32),
+                ("variances", C.c_float * 4), ("max_log_scale", C.c_float), ("clip", C.c_int32),
+                ("min_size", C.c_float), ("nms", NmsCfg)]
+
+
 class StepBuffers(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("gt_boxes", "gt_labels", "rpn_reg", "rpn_cls", "deltas", "labels",
                                           "out_boxes", "out_scores", "valid", "keep_idx")]
@@ -108,6 +114,9 @@ PROTOTYPES = {
     "tfrpn_expand_targets_host": (I, [P, P, I, I, I, P, I, P]),
     "tfrpn_roi_targets": (I, [P, P, P, P, P, I, I, I, C.POINTER(RoiTargetCfg), P, P, P, P, P, P, P, P]),
     "tfrpn_roi_head_losses": (I, [P, P, P, P, P, I, I, C.POINTER(RoiLossCfg), P, P, P, P, P]),
+    "tfrpn_roi_head_detections": (I, [P, P, P, P, P, I, I, C.POINTER(RoiDetCfg), P, P, P, P, P, P, P]),
+    "tfrpn_roi_head_detections_workspace_bytes": (C.c_size_t, [I, I, C.POINTER(RoiDetCfg)]),
+    "tfrpn_reserve_roi_head_detections": (I, [P, I, I, C.POINTER(RoiDetCfg)]),
     "tfrpn_crop_and_resize": (I, [P, I, I, I, I, P, P, I, I, I, C.c_float, P, P]),
     "tfrpn_crop_and_resize_grad_image": (I, [P, P, P, I, I, I, I, I, I, I, P, P]),
     "tfrpn_select_mask": (I, [P, P, P, I, I, I, C.c_uint64, C.c_uint64, I, I, P, P]),
