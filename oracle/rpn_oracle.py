@@ -355,6 +355,7 @@ def combined_non_max_suppression(boxes, scores, max_output_size_per_class, max_t
     total = int(max_total_size)
     out_n = total if not pad_per_class else min(total, per_class * C)
     thr = F32(iou_threshold)
+    assert F32(0) <= thr <= F32(1), "iou_threshold must be in [0, 1] (TF refuses the rest), got %r" % (iou_threshold,)
     sthr = F32(score_threshold)
     nb = np.zeros((B, out_n, 4), F32); ns = np.zeros((B, out_n), F32)
     nc = np.zeros((B, out_n), F32); nv = np.zeros((B,), np.int32)

@@ -322,6 +322,7 @@ static int proposals_host_enqueue(tfrpn_handle h, const float* rpn_reg_host, con
     if (!rpn_reg_host || !rpn_cls_host || !cfg || !out_boxes_host || !out_scores_host || !valid_host)
         return fail(TFRPN_ERR_BAD_ARG, "proposals_host: null pointer");
     if (B <= 0 || N <= 0 || cfg->post_nms_topn <= 0) return fail(TFRPN_ERR_BAD_ARG, "proposals_host: bad shape");
+    if (int rc = check_iou_threshold("proposals_host", cfg->nms_iou_threshold)) return rc;
     const int P = cfg->post_nms_topn;
     const size_t b_reg = align256((size_t)B * N * 16), b_cls = align256((size_t)B * N * 4);
     const size_t b_ob = align256((size_t)B * P * 16), b_os = align256((size_t)B * P * 4);

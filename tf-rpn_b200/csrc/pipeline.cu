@@ -703,6 +703,7 @@ static int pipe_submit(tfrpn_pipe* p, const StepArgs& a, bool acquired, bool ord
     if (do_p && (!a.rpn_cls || !a.pcfg || !a.out_boxes || !a.out_scores || !a.valid || a.pcfg->post_nms_topn <= 0))
         return fail(TFRPN_ERR_BAD_ARG, "pipeline_submit: proposal half needs rpn_cls, cfg, out_boxes, out_scores, valid");
     if (do_p && a.pcfg->pre_nms_topn <= 0) return fail(TFRPN_ERR_BAD_ARG, "pipeline_submit: pre_nms_topn must be > 0");
+    if (do_p) if (int rc = check_iou_threshold("pipeline_submit", a.pcfg->nms_iou_threshold)) return rc;
     tfrpn_handle h = p->h;
     TFRPN_ENTER(h);
     TFRPN_CHECK_ON_DEVICE(h, a.anchors_dev, "pipeline_submit: anchors_dev");

@@ -1767,6 +1767,13 @@ static IouThreshold make_threshold(float thr) {
     t.tie_up = ((nb & 1u) == 0u) ? 1 : 0;        // a tie rounds to the even mantissa
     return t;
 }
+// The IoU threshold range TF's CombinedNonMaxSuppression accepts, [0, 1] (-0.0 included).  Outside it NaN would turn
+// NMS off, and a negative threshold would let zero-area boxes suppress everything (0 > thr).
+int check_iou_threshold(const char* fn, float thr) {
+    if (!(thr >= 0.0f && thr <= 1.0f))
+        return fail(TFRPN_ERR_BAD_ARG, "%s: iou_threshold = %g must be in [0, 1]", fn, (double)thr);
+    return 0;
+}
 
 static size_t prop_smem_bytes(int n_staged, int max_out) {
     max_out = (max_out + 3) & ~3;
@@ -2264,6 +2271,7 @@ extern "C" int tfrpn_nms(tfrpn_handle h, const float* boxes, const float* scores
     if (B < 0 || K < 0) return fail(TFRPN_ERR_BAD_ARG, "nms: negative shape");
     if (cfg->max_output_size_per_class <= 0 || cfg->max_total_size <= 0)
         return fail(TFRPN_ERR_BAD_ARG, "nms: max_output_size_per_class and max_total_size must be > 0");
+    if (int rc = check_iou_threshold("nms", cfg->iou_threshold)) return rc;
     if (!aligned16(boxes) || !aligned16(out_boxes)) return fail(TFRPN_ERR_MISALIGNED, "nms: boxes must be 16-byte aligned");
     if (B == 0) return 0;
     if (!h) return fail(TFRPN_ERR_BAD_ARG, "nms: null handle");
@@ -2390,6 +2398,7 @@ extern "C" int tfrpn_proposals(tfrpn_handle h, const float* rpn_reg, const float
         return fail(TFRPN_ERR_BAD_ARG, "proposals: null pointer");
     if (B < 0 || N < 0) return fail(TFRPN_ERR_BAD_ARG, "proposals: negative shape");
     if (cfg->pre_nms_topn <= 0 || cfg->post_nms_topn <= 0) return fail(TFRPN_ERR_BAD_ARG, "proposals: topn must be > 0");
+    if (int rc = check_iou_threshold("proposals", cfg->nms_iou_threshold)) return rc;
     if (!aligned16(rpn_reg) || !aligned16(anchors) || !aligned16(out_boxes))
         return fail(TFRPN_ERR_MISALIGNED, "proposals: rpn_reg / anchors / out_boxes must be 16-byte aligned");
     if (B == 0) return 0;
@@ -2409,6 +2418,7 @@ extern "C" int tfrpn_proposals_anchor_cfg(tfrpn_handle h, const float* rpn_reg, 
         return fail(TFRPN_ERR_BAD_ARG, "proposals_anchor_cfg: null pointer");
     if (B < 0) return fail(TFRPN_ERR_BAD_ARG, "proposals_anchor_cfg: negative shape");
     if (cfg->pre_nms_topn <= 0 || cfg->post_nms_topn <= 0) return fail(TFRPN_ERR_BAD_ARG, "proposals_anchor_cfg: topn must be > 0");
+    if (int rc = check_iou_threshold("proposals_anchor_cfg", cfg->nms_iou_threshold)) return rc;
     if (!aligned16(rpn_reg) || !aligned16(out_boxes))
         return fail(TFRPN_ERR_MISALIGNED, "proposals_anchor_cfg: rpn_reg / out_boxes must be 16-byte aligned");
     AnchorGen gen;
@@ -2490,7 +2500,7 @@ int mc_check_sizes(const char* fn, int B, int K, int C, const tfrpn_nms_cfg* cfg
     if (cfg->max_output_size_per_class <= 0 || cfg->max_total_size <= 0)
         return fail(TFRPN_ERR_BAD_ARG, "%s: max_output_size_per_class and max_total_size must be > 0", fn);
     if (cfg->pre_nms_topn < 0) return fail(TFRPN_ERR_BAD_ARG, "%s: pre_nms_topn must be >= 0", fn);
-    return 0;
+    return check_iou_threshold(fn, cfg->iou_threshold);
 }
 }  // namespace tfrpn
 

@@ -182,6 +182,15 @@ def load():
     return _lib
 
 
+def iou_threshold(value, name="iou_threshold"):
+    """An NMS IoU threshold as the float32 the configuration structs carry.  Raises ValueError outside [0, 1] (NaN
+    included), the range TF's CombinedNonMaxSuppression accepts; the library refuses the same values."""
+    v = C.c_float(float(value)).value
+    if not 0.0 <= v <= 1.0:
+        raise ValueError("%s = %r must be in [0, 1]" % (name, value))
+    return v
+
+
 _STATUS = {-1: ValueError, -2: ValueError, -3: TfrpnError, -4: TfrpnError, -5: NotImplementedError}
 
 

@@ -16,8 +16,8 @@ def proposal_cfg(hyper_params, pre_nms_topn=None, post_nms_topn=None, nms_iou_th
         cfg.variances[i] = float(v)
     cfg.pre_nms_topn = int(pre_nms_topn if pre_nms_topn is not None else hyper_params.get("pre_nms_topn", 6000))
     cfg.post_nms_topn = int(post_nms_topn if post_nms_topn is not None else hyper_params["test_nms_topn"])
-    cfg.nms_iou_threshold = float(nms_iou_threshold if nms_iou_threshold is not None
-                                  else hyper_params.get("nms_iou_threshold", 0.7))
+    cfg.nms_iou_threshold = _lib.iou_threshold(nms_iou_threshold if nms_iou_threshold is not None
+                                               else hyper_params.get("nms_iou_threshold", 0.7), "nms_iou_threshold")
     cfg.clip = int(bool(clip))
     return cfg
 

@@ -62,7 +62,7 @@ def roi_head_detections(rois, cls_scores, box_deltas, valid_detections=None, *, 
     val = None if valid_detections is None else to_device(valid_detections, torch.int32, o, "valid_detections")
     if val is not None and tuple(val.shape) != (B,):
         raise ValueError("valid_detections must be (%d,), got %s" % (B, tuple(val.shape)))
-    nms = _lib.NmsCfg(int(max_output_size_per_class), int(max_total_size), float(iou_threshold),
+    nms = _lib.NmsCfg(int(max_output_size_per_class), int(max_total_size), _lib.iou_threshold(iou_threshold),
                       float(score_threshold), int(bool(pad_per_class)), int(bool(clip)), int(pre_nms_topn or 0))
     cfg = _lib.RoiDetCfg(int(Cn), int(d4.shape[2]), _SCORES[scores], (C.c_float * 4)(*[float(v) for v in variances]),
                          float(max_log_scale), int(bool(clip)), float(min_size), nms)

@@ -85,7 +85,8 @@ def non_max_suppression(pred_bboxes, pred_labels, **kwargs):
     if boxes.shape[2] != 1 or scores.shape[2] != 1:
         return _multi_class_nms(boxes, scores, kwargs, o)
     cfg = _lib.NmsCfg(int(kwargs["max_output_size_per_class"]), int(kwargs["max_total_size"]),
-                      float(kwargs.get("iou_threshold", 0.5)), float(kwargs.get("score_threshold", float("-inf"))),
+                      _lib.iou_threshold(kwargs.get("iou_threshold", 0.5)),
+                      float(kwargs.get("score_threshold", float("-inf"))),
                       int(bool(kwargs.get("pad_per_class", False))), int(bool(kwargs.get("clip_boxes", True))),
                       int(kwargs.get("pre_nms_topn") or 0))
     rows = min(cfg.max_total_size, cfg.max_output_size_per_class) if cfg.pad_per_class else cfg.max_total_size
@@ -113,7 +114,8 @@ def _multi_class_nms(boxes, scores, kwargs, o):
     if q not in (1, Cn):
         raise ValueError("pred_bboxes must be (B,K,1,4) or (B,K,C,4) for pred_labels (B,K,C); got q = %d, C = %d" % (q, Cn))
     cfg = _lib.NmsCfg(int(kwargs["max_output_size_per_class"]), int(kwargs["max_total_size"]),
-                      float(kwargs.get("iou_threshold", 0.5)), float(kwargs.get("score_threshold", float("-inf"))),
+                      _lib.iou_threshold(kwargs.get("iou_threshold", 0.5)),
+                      float(kwargs.get("score_threshold", float("-inf"))),
                       int(bool(kwargs.get("pad_per_class", False))), int(bool(kwargs.get("clip_boxes", True))),
                       int(kwargs.get("pre_nms_topn") or 0))
     if cfg.max_output_size_per_class <= 0 or cfg.max_total_size <= 0:
